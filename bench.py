@@ -53,6 +53,15 @@ WORKLOADS = {
                desc="4096 MALA chains, n=1e6 p=64 fp32 X (tcgen05 3xTF32 many-chain kernel)"),
 }
 SAMPLE_ROWS = 1_000_000     # rows of the same workload the CPU arm is timed on
+DUMP_BYTES = 64 << 20       # what --dump-outputs may write in all
+
+
+def dump_outputs(d, **arrays):
+    """--dump-outputs: each array as d/<name>.npy in float64, so that two builds run with the same
+    arguments (hence the same inputs) can be compared output for output."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def step_size(w, n):
@@ -226,10 +235,11 @@ def load_peaks():
         return {}
 
 
-def measure_c4(lr, prob, bt, w, rank, world, K, W, barrier, maxr):
+def measure_c4(lr, prob, bt, w, rank, world, K, W, barrier, maxr, dump=None):
     """Config 4: C chains in lock-step per GPU (tcgen05 3xTF32 many-chain kernel), chains sharded
     over the ranks with no collective.  A step = one MALA iteration of every chain.  Only the
-    running moments leave the device (f3): no per-step D2H of the C x p states."""
+    running moments leave the device (f3): no per-step D2H of the C x p states.
+    dump: directory for this rank's outputs of the timed run (pooled moments, accepted counts)."""
     n, p, C = w["n"], w["p"], w["chains"]
     c_lo, c_hi = (rank * C) // world, ((rank + 1) * C) // world
     Cl = c_hi - c_lo
@@ -244,6 +254,8 @@ def measure_c4(lr, prob, bt, w, rank, world, K, W, barrier, maxr):
     cnt, mean, cov = prob.moments(pooled=True)                                                     # O(p^2) out, once
     dt = maxr(time.perf_counter() - t0)
     inf1 = prob.info()
+    if dump:
+        dump_outputs(dump, moments_count=[cnt], moments_mean=mean, moments_cov=cov, accepted=acc)
     peaks = load_peaks()
     value = C * K / dt
     flops = 4.0 * n * p * Cl * (K + 1)             # algorithmic (1-pass) flops on this rank, incl. the init evaluation
@@ -295,7 +307,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--deterministic", action="store_true", help="static fixed-order kernel instead of drive mode")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (float64, rank 0): "
+                         "the sample matrix (its last rows if above 32 MB), final state and lpost, and the number of "
+                         "timed steps accepted; for c4 the pooled moments and each chain's accepted timed steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
     w = dict(WORKLOADS[args.workload])
     if args.n:
         w["n"] = args.n
@@ -363,7 +383,8 @@ def main():
         # --workload c4 as the headline line (development / profiles); the driver's line is c3
         prob = lr.Problem(local, deterministic=args.deterministic)
         bt = prob.gen_synthetic(n, p, mode=w["mode"], seed=42)
-        r = measure_c4(lr, prob, bt, w, rank, world, max(K, 40), max(W, 10), barrier, maxr)
+        r = measure_c4(lr, prob, bt, w, rank, world, K, max(W, 10), barrier, maxr,
+                       dump=args.dump_outputs if rank == 0 else None)
         if rank == 0:
             line = {"metric": metric, "value": r["chain_iters_per_s"], "unit": "evals/s", "n_gpus": world, "steps": r["steps"],
                     "warmup": r["warmup"], "ms_per_step": r["ms_per_step"], "higher_is_better": True,
@@ -460,6 +481,10 @@ def main():
             print(json.dumps({"error": "ranks disagree on the sample matrix / final state", "digest": digest}))
         finish()
         return 1
+    if args.dump_outputs and rank == 0:
+        keep = DUMP_BYTES // 2 // (8 * p)
+        dump_outputs(args.dump_outputs, samples=out[-keep:], final_x=x_fin, final_lpost=[lp_fin],
+                     accepted=[acc1.value - acc.value])
 
     # ---- e2e through the public API: host state in, host sample out, every step
     x = out[-1].copy()

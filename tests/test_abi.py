@@ -52,25 +52,41 @@ def test_key_child_is_host_arithmetic_and_matches_the_philox_spec():
     assert J.split(42, 4) == [lib.lrb_key_child(42, i) for i in range(4)]
 
 
+NO_GPU_CHECK = """
+import sys
+sys.path.insert(0, sys.argv[1])
+import numpy as np
+import pytest
+import logreg_b200 as lr
+from logreg_b200 import _native as N
+try:
+    have = N.device_count() > 0
+except lr.LogregB200Error as e:
+    have = False
+    assert e.code == N.E_NO_DEVICE
+    assert "no CPU fallback" in str(e)
+assert not have
+with pytest.raises(lr.LogregB200Error):
+    lr.Problem(0)
+with pytest.raises(lr.LogregB200Error):
+    lr.bind_data(np.ones((4, 2)), np.zeros(4, dtype=np.float32))
+with pytest.raises(lr.LogregB200Error, match="bind_data"):
+    lr.use(None)
+    lr.lpost(np.zeros(2))
+print("NO_GPU_OK")
+"""
+
+
 def test_no_gpu_means_loud_failure():
-    """On a box without a CUDA device the product path must raise, not fall back."""
-    import logreg_b200 as lr
+    """On a box without a CUDA device the product path must raise, not fall back.  Runs in a child
+    process that sees no device (CUDA_VISIBLE_DEVICES empty), so it also runs where a GPU is present."""
+    import subprocess
+    import sys
     from logreg_b200 import _native as N
-    try:
-        have = N.device_count() > 0
-    except lr.LogregB200Error as e:
-        have = False
-        assert e.code == N.E_NO_DEVICE
-        assert "no CPU fallback" in str(e)
-    if have:
-        pytest.skip("a CUDA device is present")
-    with pytest.raises(lr.LogregB200Error):
-        lr.Problem(0)
-    with pytest.raises(lr.LogregB200Error):
-        lr.bind_data(np.ones((4, 2)), np.zeros(4, dtype=np.float32))
-    with pytest.raises(lr.LogregB200Error, match="bind_data"):
-        lr.use(None)
-        lr.lpost(np.zeros(2))
+    N.load()
+    r = subprocess.run([sys.executable, "-c", NO_GPU_CHECK, ROOT], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0 and "NO_GPU_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_product_code_never_imports_the_oracle():

@@ -23,10 +23,23 @@ def test_load_pima_formats(pima, tmp_path):
     X2, y2 = load_pima(path)
     np.testing.assert_array_equal(X2, pima["X"])
     np.testing.assert_array_equal(y2, pima["y"])
-    if os.path.exists("/root/reference/pima.parquet"):
-        X3, y3 = load_pima("/root/reference/pima.parquet")
-        np.testing.assert_array_equal(X3, pima["X"])
-        np.testing.assert_array_equal(y3, pima["y"])
+    # the reference's pima.parquet (R/create-dataset.R writes MASS::Pima.tr) in the schema recorded in
+    # SURVEY.md (data files): five int32 and two float64 covariates, then `type`, a Yes/No category
+    import pandas as pd
+    schema = {"npreg": "int32", "glu": "int32", "bp": "int32", "skin": "int32", "bmi": "float64", "ped": "float64",
+              "age": "int32"}
+    cov = pima["X"][:, 1:]
+    ints = [j for j, t in enumerate(schema.values()) if t == "int32"]
+    np.testing.assert_array_equal(cov[:, ints], np.round(cov[:, ints]))     # the int32 columns hold integers
+    df = pd.DataFrame({name: cov[:, j].astype(t) for j, (name, t) in enumerate(schema.items())})
+    df["type"] = pd.Categorical(np.where(pima["y"] == 1, "Yes", "No"), categories=["No", "Yes"])
+    df.to_parquet(tmp_path / "pima.parquet")
+    back = pd.read_parquet(tmp_path / "pima.parquet")
+    assert {c: str(t) for c, t in back.dtypes.items()} == dict(schema, type="category")
+    X3, y3 = load_pima(tmp_path / "pima.parquet")
+    assert X3.flags["F_CONTIGUOUS"] and y3.dtype == np.float32
+    np.testing.assert_array_equal(X3, pima["X"])
+    np.testing.assert_array_equal(y3, pima["y"])
 
 
 def test_describe_matches_scipy_and_save_roundtrip(tmp_path):
