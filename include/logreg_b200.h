@@ -236,6 +236,27 @@ int lrb_debug_chol_solve(double* A, int ld, int p, const double* pscale, const d
 /* lprior alone (fit-np-ul.py:33-34; no pass over X). beta: C x p host; out: C. */
 int lrb_lprior(lrb_handle* h, const double* beta, int C, double* out);
 
+/* ---- posterior predictive summaries and WAIC over posterior draws ------------------------
+ * One pass over the bound rows for all S draws (draws: S x p float64, host, row-major).  With
+ * eta_is = x_i . beta_s and l_is = log p(y_i | beta_s), per row i (each output n doubles, may be
+ * NULL: a NULL output is neither computed into HBM nor copied):
+ *   prob_mean[i] = mean_s sigmoid(eta_is)     prob_sd[i] = sd_s sigmoid(eta_is)   (ddof 1)
+ *   lppd[i]      = log mean_s exp(l_is)       p_waic[i]  = var_s l_is             (ddof 1)
+ * (prob_sd and p_waic are NaN for S = 1.)  `location` (LRB_HOST / LRB_DEVICE) says where the four
+ * output pointers live.  totals (may be NULL): lppd = sum lppd[i], p_waic = sum p_waic[i],
+ * elpd_waic = lppd - p_waic, se_elpd_waic = sqrt(n var_i(lppd[i] - p_waic[i])) (ddof 1).
+ * Arithmetic of the mode: eta in float32 (FP32, beta rounded to float) or float64 (FP64); the
+ * statistics are accumulated in float64.  Results are bit-reproducible for a fixed shape.  The
+ * sampler state and a paused chain are untouched.  Row-sharded handles: LRB_E_UNSUPPORTED. */
+typedef struct lrb_predictive_totals {
+  int64_t n;            /* rows scored (this handle's rows) */
+  int64_t draws;        /* S */
+  double lppd, p_waic, elpd_waic, se_elpd_waic;
+} lrb_predictive_totals;   /* 48 bytes */
+int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int location,
+                   double* prob_mean, double* prob_sd, double* lppd, double* p_waic,
+                   lrb_predictive_totals* totals);
+
 /* ---- samplers: mcmc(init, kernel, thin, iters) -------------------------------
  * Runs the whole chain on the device (no per-iteration host round trip):
  * replaces `mcmc` (fit-numpy.py:64-79, fit-np-ul.py:70-84) driving `mhKernel` /

@@ -47,6 +47,11 @@ class Info(C.Structure):
                 ("eval_launches", C.c_int64)]
 
 
+class PredictiveTotals(C.Structure):
+    _fields_ = [("n", C.c_int64), ("draws", C.c_int64), ("lppd", C.c_double), ("p_waic", C.c_double),
+                ("elpd_waic", C.c_double), ("se_elpd_waic", C.c_double)]
+
+
 _vp, _i, _i64, _u64 = C.c_void_p, C.c_int, C.c_int64, C.c_uint64
 _dp = C.POINTER(C.c_double)
 
@@ -67,6 +72,7 @@ SIGNATURES = {
     "lrb_eval": (_i, [_vp, _dp, _i, _i, _dp, _dp, _dp]),
     "lrb_eval_device": (_i, [_vp, _vp, _vp, _i]),
     "lrb_lprior": (_i, [_vp, _dp, _i, _dp]),
+    "lrb_predictive": (_i, [_vp, _dp, _i64, _i, _vp, _vp, _vp, _vp, C.POINTER(PredictiveTotals)]),
     "lrb_map": (_i, [_vp, _dp, C.c_double, _i, _dp, C.POINTER(MapInfo)]),
     "lrb_hessian": (_i, [_vp, _dp, _dp]),
     "lrb_debug_chol_solve": (_i, [_dp, _i, _i, _dp, _dp, _dp]),

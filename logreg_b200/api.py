@@ -29,6 +29,7 @@ from ._native import LogregB200Error
 
 _MODES = {"fp64": N.MODE_FP64, "fp32": N.MODE_FP32, N.MODE_FP64: N.MODE_FP64, N.MODE_FP32: N.MODE_FP32}
 _REPLAY_CHUNK_BYTES = 64 << 20
+_PREDICTIVE_OUTPUTS = ("prob_mean", "prob_sd", "lppd", "p_waic")   # argument order of lrb_predictive
 
 
 def _vec(v, p, name):
@@ -251,6 +252,44 @@ class Problem:
         H = np.empty((self.p, self.p))
         self._ck(self._lib.lrb_hessian(self._h, N.as_dp(b), N.as_dp(H)))
         return H
+
+    # ------------------------------------------------------------ posterior predictive / WAIC
+    def predictive(self, draws, pointwise=True, device_out=False):
+        """Posterior predictive summaries of the bound rows over posterior draws, one pass over X
+        on the device (lrb_predictive). draws: (S, p), or (C, iters, p) from run_chains (flattened).
+
+        Returns a dict with the totals lppd, p_waic, elpd_waic, se_elpd_waic, n and draws (= S), and
+        with pointwise=True also out["pointwise"] = {prob_mean, prob_sd, lppd, p_waic}: per-row
+        arrays of length n (the mean and sd of sigmoid(x.beta) over the draws, log of the mean
+        predictive density of y, variance of the log density; sd and variance have ddof 1 and are
+        NaN for S = 1). They are NumPy arrays, or float64 torch CUDA tensors with device_out=True.
+        The sampler state, a paused chain and the cached evaluation are left as they were."""
+        return self._predictive(draws, _PREDICTIVE_OUTPUTS if pointwise else (), device_out)
+
+    def _predictive(self, draws, outputs, device_out):
+        B = np.asarray(draws, dtype=np.float64)
+        if B.ndim == 3:
+            B = B.reshape(-1, B.shape[-1])
+        if B.ndim != 2 or (self.p and B.shape[1] != self.p):
+            raise LogregB200Error(N.E_BAD_ARG, f"draws must have shape (S, {self.p}) or (C, iters, {self.p}), "
+                                               f"got {np.shape(draws)}")
+        B = np.ascontiguousarray(B)
+        if device_out:
+            import torch
+            dev = torch.device("cuda", self.device)
+            bufs = {k: torch.empty(self.n, dtype=torch.float64, device=dev) for k in outputs}
+            torch.cuda.current_stream(dev).synchronize()
+            ptr, loc = (lambda t: t.data_ptr()), N.DEVICE
+        else:
+            bufs = {k: np.empty(self.n) for k in outputs}
+            ptr, loc = (lambda a: a.ctypes.data), N.HOST
+        ptrs = [C.c_void_p(ptr(bufs[k])) if k in bufs else None for k in _PREDICTIVE_OUTPUTS]
+        tot = N.PredictiveTotals()
+        self._ck(self._lib.lrb_predictive(self._h, N.as_dp(B), B.shape[0], loc, *ptrs, C.byref(tot)))
+        out = {k: getattr(tot, k) for k, _ in N.PredictiveTotals._fields_}
+        if outputs:
+            out["pointwise"] = bufs
+        return out
 
     # ------------------------------------------------------------ sampler runs
     def _params(self, k, seed, rng, init_lpost, flags=0, t0=0):

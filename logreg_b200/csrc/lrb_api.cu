@@ -21,6 +21,7 @@
 #include "eval_persist_kernel.cuh"
 #include "eval_tc_kernel.cuh"
 #include "newton.cuh"
+#include "predictive.cuh"
 #include "sampler.cuh"
 
 using namespace lrb;
@@ -1092,6 +1093,114 @@ extern "C" int lrb_lprior(lrb_handle* h, const double* beta, int C, double* out)
   h->kernel_launches++;
   CK(h, cudaMemcpyAsync(out, dout, (size_t)C * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaStreamSynchronize(h->stream));
+  return LRB_OK;
+}
+
+// ============================================================ posterior predictive / WAIC
+namespace {
+
+using PredFn = void (*)(const PredictiveArgs);
+
+template <typename T, int P>
+PredFn predictive_for(size_t& smem) {
+  smem = predictive_smem<T, P>();
+  return predictive_kernel<T, P>;
+}
+
+template <typename T>
+PredFn pick_predictive(int P, size_t& smem) {
+  switch (P) {
+    case 8: return predictive_for<T, 8>(smem);
+    case 16: return predictive_for<T, 16>(smem);
+    case 32: return predictive_for<T, 32>(smem);
+    case 64: return predictive_for<T, 64>(smem);
+    case 128: return predictive_for<T, 128>(smem);
+    case 256: return predictive_for<T, 256>(smem);
+  }
+  return nullptr;
+}
+
+// draws (S x p, float64, row-major, host) -> dst: P x Spad in the mode's dtype, k-major, zero padded
+template <typename T>
+int upload_draws(lrb_handle* h, void* dst, const double* draws, long long S, long long Spad) {
+  std::vector<T> bt((size_t)h->P * Spad, (T)0);
+  for (long long s = 0; s < S; ++s)
+    for (int k = 0; k < h->p; ++k) bt[(size_t)k * Spad + s] = (T)draws[(size_t)s * h->p + k];
+  CK(h, cudaMemcpyAsync(dst, bt.data(), bt.size() * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));   // bt is pageable host memory and dies here
+  return LRB_OK;
+}
+
+}  // namespace
+
+extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int location, double* prob_mean,
+                              double* prob_sd, double* lppd, double* p_waic, lrb_predictive_totals* totals) {
+  if (!h) return fail(nullptr, LRB_E_BAD_ARG, "handle is NULL");
+  if (!h->bound) return fail(h, LRB_E_STATE, "lrb_predictive before lrb_bind_data / lrb_gen_synthetic");
+  if (!draws || S < 1) return fail(h, LRB_E_BAD_ARG, "draws is NULL or S < 1 (S=%lld)", (long long)S);
+  if (S > (1ll << 30)) return fail(h, LRB_E_BAD_ARG, "S=%lld draws exceeds 2^30", (long long)S);
+  if (location != LRB_HOST && location != LRB_DEVICE) return fail(h, LRB_E_BAD_ARG, "bad location %d", location);
+  if (h->world > 1)
+    return fail(h, LRB_E_UNSUPPORTED, "lrb_predictive works on single-GPU handles only: this handle is rank %d of a "
+                "row-sharded group of %d, and its per-shard totals would need a collective", h->rank, h->world);
+  if (use_device(h)) return LRB_E_CUDA;
+  const bool fp32 = h->mode == LRB_MODE_FP32;
+  const int P = h->P;
+  size_t smem = 0;
+  PredFn fn = fp32 ? pick_predictive<float>(P, smem) : pick_predictive<double>(P, smem);
+  if (!fn) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", P);
+  CK(h, cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kBlock, smem));
+  if (occ < 1) return fail(h, LRB_E_CUDA, "predictive kernel does not fit an SM");
+  const long long ntiles = (h->n + kPredRows - 1) / kPredRows;
+  const int grid = (int)std::min<long long>((long long)h->sms * occ, ntiles);
+  const long long Spad = (S + kPredDraws - 1) / kPredDraws * kPredDraws;
+
+  // scratch: draws, CTA partials, totals, ticket; per-row outputs on the device when the caller's are on the host
+  DevTmp dB, work, out[4];
+  const size_t es = fp32 ? 4 : 8;
+  CK(h, dB.alloc((size_t)P * Spad * es));
+  int rc = fp32 ? upload_draws<float>(h, dB.p, draws, S, Spad) : upload_draws<double>(h, dB.p, draws, S, Spad);
+  if (rc) return rc;
+  const size_t wdoubles = (size_t)grid * kPredPartial + kPredTotals;
+  CK(h, work.alloc(wdoubles * sizeof(double) + sizeof(unsigned int)));
+  unsigned int* ticket = reinterpret_cast<unsigned int*>(work.as<double>() + wdoubles);
+  CK(h, cudaMemsetAsync(ticket, 0, sizeof(unsigned int), h->stream));
+  double* user[4] = {prob_mean, prob_sd, lppd, p_waic};
+  double* dev[4] = {};
+  for (int k = 0; k < 4; ++k) {
+    if (!user[k]) continue;
+    if (location == LRB_DEVICE) { dev[k] = user[k]; continue; }
+    CK(h, out[k].alloc((size_t)h->n * sizeof(double)));
+    dev[k] = out[k].as<double>();
+  }
+
+  PredictiveArgs a{};
+  a.X = h->X; a.y = h->y; a.n = h->n;
+  a.B = dB.p; a.S = S; a.Spad = Spad;
+  a.prob_mean = dev[0]; a.prob_sd = dev[1]; a.lppd = dev[2]; a.p_waic = dev[3];
+  a.partials = work.as<double>();
+  a.ticket = ticket;
+  a.totals = work.as<double>() + (size_t)grid * kPredPartial;
+  fn<<<grid, kBlock, smem, h->stream>>>(a);
+  CK(h, cudaGetLastError());
+  h->kernel_launches++;
+
+  double tot[kPredTotals];
+  CK(h, cudaMemcpyAsync(tot, a.totals, sizeof tot, cudaMemcpyDeviceToHost, h->stream));
+  if (location == LRB_HOST)
+    for (int k = 0; k < 4; ++k)
+      if (user[k]) CK(h, cudaMemcpyAsync(user[k], dev[k], (size_t)h->n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(h, cudaStreamSynchronize(h->stream));   // the temporaries die with this scope
+  if (totals) {
+    totals->n = h->n;
+    totals->draws = S;
+    totals->lppd = tot[0];
+    totals->p_waic = tot[1];
+    totals->elpd_waic = tot[2];
+    totals->se_elpd_waic = tot[3];
+  }
   return LRB_OK;
 }
 

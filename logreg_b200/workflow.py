@@ -1,5 +1,6 @@
 """The steps either side of the hot path (SURVEY.md 8f), as thin host helpers around the
-device kernels: data ingest (f2), MAP initialisation (f1), output + summaries (f3).
+device kernels: data ingest (f2), MAP initialisation (f1), output + summaries (f3), and what a
+fitted model is for: predictions and WAIC / held-out lppd over the posterior draws.
 
 Reference lines mirrored (paths relative to the reference root):
     load_pima       Python/fit-numpy.py:12-19 (parquet -> X with a ones column, y float32)
@@ -12,6 +13,13 @@ Reference lines mirrored (paths relative to the reference root):
                     Dex/djwutils.dx:97-103 meanAndCovariance)
     save_samples    Python/fit-numpy.py:89-90  DataFrame(out, columns=b0..).to_parquet(...)
     describe        Python/fit-numpy.py:92-96  scipy.stats.describe(out): mean / variance
+
+Beyond the reference (which stops at the samples), over S posterior draws on the device
+(lrb_predictive, one pass over the bound rows for all draws):
+    waic            elpd_waic, p_waic, lppd, se_elpd_waic of the rows bound to a Problem: WAIC on the
+                    training rows, or the held-out lppd on a Problem bound to test rows
+    waic_from_pointwise  the same totals from per-row lppd / p_waic arrays, e.g. of several Problems
+    predict_proba   posterior mean and sd of P(y = 1 | x) for unlabelled rows
 """
 from __future__ import annotations
 
@@ -107,6 +115,47 @@ def effective_sample_size(mat, max_lag=200):
             s += r
         out[j] = n / (1 + 2 * s)
     return out
+
+
+_WAIC_KEYS = ("elpd_waic", "p_waic", "lppd", "se_elpd_waic", "n", "draws")
+
+
+def waic(problem, draws):
+    """WAIC of the rows bound to `problem` over posterior draws (S, p) or (C, iters, p):
+    {elpd_waic, p_waic, lppd, se_elpd_waic, n, draws}, with lppd = sum_i log mean_s p(y_i | beta_s),
+    p_waic = sum_i var_s log p(y_i | beta_s), elpd_waic = lppd - p_waic and
+    se_elpd_waic = sqrt(n var_i(elpd_i)) as R's loo package reports them. Bound to held-out rows,
+    `lppd` is the held-out log pointwise predictive density. Nothing per row leaves the device."""
+    t = problem.predictive(draws, pointwise=False)
+    return {k: t[k] for k in _WAIC_KEYS}
+
+
+def waic_from_pointwise(lppd, p_waic, draws):
+    """The totals of `waic` from per-row arrays (predictive(...)["pointwise"]["lppd"] / ["p_waic"]),
+    e.g. concatenated over Problems holding parts of one data set; `draws` is S."""
+    lppd = np.asarray(lppd, dtype=np.float64)
+    p_waic = np.asarray(p_waic, dtype=np.float64)
+    elpd = lppd - p_waic
+    n = elpd.shape[0]
+    return {"elpd_waic": float(elpd.sum()), "p_waic": float(p_waic.sum()), "lppd": float(lppd.sum()),
+            "se_elpd_waic": float(np.sqrt(n * elpd.var(ddof=1))) if n > 1 else float("nan"),
+            "n": n, "draws": int(draws)}
+
+
+def predict_proba(X_new, draws, mode="fp64", device=0):
+    """Posterior mean and sd (ddof 1) of P(y = 1 | x) = sigmoid(x.beta) over the draws for the
+    rows of X_new (n_new, p): returns (prob_mean, prob_sd) as NumPy arrays. X_new is bound to a
+    fresh Problem with all-zero labels; the labels are unused (only the two probability outputs
+    are requested)."""
+    from .api import Problem
+    X_new = np.asarray(X_new)
+    prob = Problem(device)
+    try:
+        prob.bind_data(X_new, np.zeros(X_new.shape[0], dtype=np.float32), mode=mode)
+        pw = prob._predictive(draws, ("prob_mean", "prob_sd"), device_out=False)["pointwise"]
+    finally:
+        prob.close()
+    return pw["prob_mean"], pw["prob_sd"]
 
 
 def save_samples(mat, path):
