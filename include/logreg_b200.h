@@ -257,6 +257,43 @@ int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int location,
                    double* prob_mean, double* prob_sd, double* lppd, double* p_waic,
                    lrb_predictive_totals* totals);
 
+/* ---- PSIS-LOO cross-validation and the pointwise log-likelihood over posterior draws ---------
+ * Pareto-smoothed importance-sampling leave-one-out (Vehtari, Simpson, Gelman, Yao & Gabry 2024),
+ * exactly R's loo package: psis() with r_eff = 1 (generalized Pareto fit of Zhang & Stephens 2009
+ * with loo's weak prior and wip adjustment; tail length M = ceil(min(0.2 S, 3 sqrt(S))); no
+ * smoothing and k-hat = +inf when M < 5, i.e. S < 21, or the tail is constant).  Per row i, with
+ * l_is = log p(y_i | beta_s) and lw_i the log weights of the log ratios -l_i:
+ *   elpd_loo[i] = log sum_s exp(lw_is + l_is) - log sum_s exp(lw_is)
+ *   p_loo[i]    = lppd_i - elpd_loo[i]       (lppd_i = log mean_s exp(l_is))
+ *   pareto_k[i] = k-hat of the row (the reliability diagnostic of elpd_loo[i])
+ * draws: S x p float64, host, row-major; 1 <= S <= 2^21.  Each per-row output (n doubles) may be
+ * NULL; `location` (LRB_HOST / LRB_DEVICE) says where they live.  totals (may be NULL):
+ * elpd_loo and p_loo summed over the rows, se_* = sqrt(n var_i(.)) (ddof 1), looic = -2 elpd_loo,
+ * k_threshold = min(1 - 1/log10 S, 0.7) (loo >= 2.7), k_max and n_k_high = #{i : pareto_k[i] >
+ * k_threshold}.  Rows are scored in chunks through a bounded scratch matrix; results are
+ * bit-reproducible for a fixed shape.  The sampler state and a paused chain are untouched.
+ * Row-sharded handles: LRB_E_UNSUPPORTED.
+ * Benchmark switch: with the environment variable LRB_LOO_STAGE1_ONLY set, only the
+ * log-likelihood stage runs (to time it alone); every per-row output and every floating-point
+ * total is then NaN and n_k_high is -1.  LRB_LOO_CHUNK_MB overrides the 64 MB scratch budget. */
+typedef struct lrb_loo_totals {
+  int64_t n, draws;
+  double elpd_loo, se_elpd_loo, p_loo, se_p_loo, looic;
+  double k_threshold, k_max;
+  int64_t n_k_high;
+} lrb_loo_totals;                                   /* 80 bytes */
+int lrb_loo(lrb_handle* h, const double* draws, int64_t S, int location,
+            double* elpd_loo, double* p_loo, double* pareto_k, lrb_loo_totals* totals);
+/* l_is = log p(y_i | beta_s) for the bound rows [row0, row0 + nrows) and all S draws (1 <= S <=
+ * 2^21): out is nrows x S, row-major, float64, on the host or the device (`location`); the matrix
+ * loo::loo() and ArviZ take, transposed.  Host output is copied chunk by chunk (bounded device
+ * memory).  Arithmetic of the mode, as lrb_predictive.  Row-sharded handles: LRB_E_UNSUPPORTED. */
+int lrb_loglik(lrb_handle* h, const double* draws, int64_t S, int64_t row0, int64_t nrows,
+               int location, double* out);          /* out: nrows x S, row-major, float64 */
+/* loo's psis() of one row on the host, the same formulas psis_kernel runs (no GPU needed):
+ * log_ratios[S] -> log_weights[S] (smoothed, truncated at the largest raw weight) and k-hat. */
+int lrb_debug_psis(const double* log_ratios, int64_t S, double* log_weights, double* khat);
+
 /* ---- samplers: mcmc(init, kernel, thin, iters) -------------------------------
  * Runs the whole chain on the device (no per-iteration host round trip):
  * replaces `mcmc` (fit-numpy.py:64-79, fit-np-ul.py:70-84) driving `mhKernel` /

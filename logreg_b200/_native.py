@@ -52,6 +52,12 @@ class PredictiveTotals(C.Structure):
                 ("elpd_waic", C.c_double), ("se_elpd_waic", C.c_double)]
 
 
+class LooTotals(C.Structure):
+    _fields_ = [("n", C.c_int64), ("draws", C.c_int64), ("elpd_loo", C.c_double), ("se_elpd_loo", C.c_double),
+                ("p_loo", C.c_double), ("se_p_loo", C.c_double), ("looic", C.c_double),
+                ("k_threshold", C.c_double), ("k_max", C.c_double), ("n_k_high", C.c_int64)]
+
+
 _vp, _i, _i64, _u64 = C.c_void_p, C.c_int, C.c_int64, C.c_uint64
 _dp = C.POINTER(C.c_double)
 
@@ -73,6 +79,9 @@ SIGNATURES = {
     "lrb_eval_device": (_i, [_vp, _vp, _vp, _i]),
     "lrb_lprior": (_i, [_vp, _dp, _i, _dp]),
     "lrb_predictive": (_i, [_vp, _dp, _i64, _i, _vp, _vp, _vp, _vp, C.POINTER(PredictiveTotals)]),
+    "lrb_loo": (_i, [_vp, _dp, _i64, _i, _vp, _vp, _vp, C.POINTER(LooTotals)]),
+    "lrb_loglik": (_i, [_vp, _dp, _i64, _i64, _i64, _i, _vp]),
+    "lrb_debug_psis": (_i, [_dp, _i64, _dp, _dp]),
     "lrb_map": (_i, [_vp, _dp, C.c_double, _i, _dp, C.POINTER(MapInfo)]),
     "lrb_hessian": (_i, [_vp, _dp, _dp]),
     "lrb_debug_chol_solve": (_i, [_dp, _i, _i, _dp, _dp, _dp]),

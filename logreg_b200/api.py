@@ -14,6 +14,11 @@ this backend with
     from logreg_b200 import *          # instead of defining ll/lprior/lpost/glp/...Kernel/mcmc
     bind_data(X, y, pscale)            # the one extra line: closures cannot be imported
 
+Beyond the reference, a Problem scores its bound rows under posterior draws on the device:
+`predictive` (posterior predictive probabilities, lppd, WAIC), `loo` (PSIS-LOO: elpd_loo, p_loo and
+the Pareto k-hat of every row, as R's loo package computes them) and `loglik` (the pointwise
+log-likelihood matrix).
+
 Everything numeric runs on the GPU; without a CUDA device every call raises
 `LogregB200Error` (there is no CPU fallback).
 """
@@ -30,6 +35,7 @@ from ._native import LogregB200Error
 _MODES = {"fp64": N.MODE_FP64, "fp32": N.MODE_FP32, N.MODE_FP64: N.MODE_FP64, N.MODE_FP32: N.MODE_FP32}
 _REPLAY_CHUNK_BYTES = 64 << 20
 _PREDICTIVE_OUTPUTS = ("prob_mean", "prob_sd", "lppd", "p_waic")   # argument order of lrb_predictive
+_LOO_OUTPUTS = ("elpd_loo", "p_loo", "pareto_k")                    # argument order of lrb_loo
 
 
 def _vec(v, p, name):
@@ -267,22 +273,8 @@ class Problem:
         return self._predictive(draws, _PREDICTIVE_OUTPUTS if pointwise else (), device_out)
 
     def _predictive(self, draws, outputs, device_out):
-        B = np.asarray(draws, dtype=np.float64)
-        if B.ndim == 3:
-            B = B.reshape(-1, B.shape[-1])
-        if B.ndim != 2 or (self.p and B.shape[1] != self.p):
-            raise LogregB200Error(N.E_BAD_ARG, f"draws must have shape (S, {self.p}) or (C, iters, {self.p}), "
-                                               f"got {np.shape(draws)}")
-        B = np.ascontiguousarray(B)
-        if device_out:
-            import torch
-            dev = torch.device("cuda", self.device)
-            bufs = {k: torch.empty(self.n, dtype=torch.float64, device=dev) for k in outputs}
-            torch.cuda.current_stream(dev).synchronize()
-            ptr, loc = (lambda t: t.data_ptr()), N.DEVICE
-        else:
-            bufs = {k: np.empty(self.n) for k in outputs}
-            ptr, loc = (lambda a: a.ctypes.data), N.HOST
+        B = self._draws(draws)
+        bufs, ptr, loc = self._row_outputs(outputs, (self.n,), device_out)
         ptrs = [C.c_void_p(ptr(bufs[k])) if k in bufs else None for k in _PREDICTIVE_OUTPUTS]
         tot = N.PredictiveTotals()
         self._ck(self._lib.lrb_predictive(self._h, N.as_dp(B), B.shape[0], loc, *ptrs, C.byref(tot)))
@@ -290,6 +282,59 @@ class Problem:
         if outputs:
             out["pointwise"] = bufs
         return out
+
+    # ------------------------------------------------------------ PSIS-LOO / pointwise log-likelihood
+    def _draws(self, draws):
+        B = np.asarray(draws, dtype=np.float64)
+        if B.ndim == 3:
+            B = B.reshape(-1, B.shape[-1])
+        if B.ndim != 2 or (self.p and B.shape[1] != self.p):
+            raise LogregB200Error(N.E_BAD_ARG, f"draws must have shape (S, {self.p}) or (C, iters, {self.p}), "
+                                               f"got {np.shape(draws)}")
+        return np.ascontiguousarray(B)
+
+    def loo(self, draws, pointwise=True, device_out=False):
+        """Pareto-smoothed importance-sampling leave-one-out cross-validation of the bound rows over
+        posterior draws (lrb_loo; R's loo::loo() with r_eff = 1). draws: (S, p), or (C, iters, p)
+        from run_chains (flattened); 1 <= S <= 2^21.
+
+        Returns a dict with the totals elpd_loo, se_elpd_loo, p_loo, se_p_loo, looic, se_looic
+        (= 2 se_elpd_loo), k_threshold (= min(1 - 1/log10 S, 0.7)), k_max, n_k_high (rows whose
+        pareto_k exceeds k_threshold: their elpd_loo is unreliable), n and draws, and with
+        pointwise=True also out["pointwise"] = {elpd_loo, p_loo, pareto_k}: per-row arrays of length
+        n, NumPy arrays or float64 torch CUDA tensors with device_out=True. The sampler state, a paused
+        chain and the cached evaluation are left as they were."""
+        B = self._draws(draws)
+        bufs, ptr, loc = self._row_outputs(_LOO_OUTPUTS if pointwise else (), (self.n,), device_out)
+        ptrs = [C.c_void_p(ptr(bufs[k])) if k in bufs else None for k in _LOO_OUTPUTS]
+        tot = N.LooTotals()
+        self._ck(self._lib.lrb_loo(self._h, N.as_dp(B), B.shape[0], loc, *ptrs, C.byref(tot)))
+        out = {k: getattr(tot, k) for k, _ in N.LooTotals._fields_}
+        out["se_looic"] = 2.0 * out["se_elpd_loo"]
+        if pointwise:
+            out["pointwise"] = bufs
+        return out
+
+    def loglik(self, draws, row0=0, nrows=None, device_out=False):
+        """log p(y_i | beta_s) for the bound rows row0 .. row0 + nrows - 1 and every draw (lrb_loglik):
+        an (nrows, S) float64 array (a torch CUDA tensor with device_out=True). Its transpose is the
+        S x n matrix R's loo::loo() and ArviZ take. 1 <= S <= 2^21."""
+        B = self._draws(draws)
+        nrows = self.n - int(row0) if nrows is None else int(nrows)
+        bufs, ptr, loc = self._row_outputs(("L",), (max(nrows, 0), B.shape[0]), device_out)
+        self._ck(self._lib.lrb_loglik(self._h, N.as_dp(B), B.shape[0], int(row0), nrows, loc,
+                                      C.c_void_p(ptr(bufs["L"]))))
+        return bufs["L"]
+
+    def _row_outputs(self, names, shape, device_out):
+        """float64 output buffers on the host or this Problem's GPU, and how to pass them."""
+        if device_out:
+            import torch
+            dev = torch.device("cuda", self.device)
+            bufs = {k: torch.empty(shape, dtype=torch.float64, device=dev) for k in names}
+            torch.cuda.current_stream(dev).synchronize()
+            return bufs, (lambda t: t.data_ptr()), N.DEVICE
+        return {k: np.empty(shape) for k in names}, (lambda a: a.ctypes.data), N.HOST
 
     # ------------------------------------------------------------ sampler runs
     def _params(self, k, seed, rng, init_lpost, flags=0, t0=0):

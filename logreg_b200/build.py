@@ -21,7 +21,7 @@ LIB = os.path.join(LIBDIR, "liblogreg_b200.so")
 STAMP = os.path.join(LIBDIR, "liblogreg_b200.srchash")
 
 SOURCES = ["lrb_api.cu"]
-HEADERS = ["common.cuh", "sampler.cuh", "eval_kernel.cuh", "eval_mc_kernel.cuh", "eval_tc_kernel.cuh", "eval_persist_kernel.cuh", "newton.cuh", "data.cuh", "predictive.cuh"]
+HEADERS = ["common.cuh", "sampler.cuh", "eval_kernel.cuh", "eval_mc_kernel.cuh", "eval_tc_kernel.cuh", "eval_persist_kernel.cuh", "newton.cuh", "data.cuh", "predictive.cuh", "loo.cuh"]
 
 
 def nccl_include() -> str:

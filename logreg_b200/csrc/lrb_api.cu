@@ -20,6 +20,7 @@
 #include "eval_mc_kernel.cuh"
 #include "eval_persist_kernel.cuh"
 #include "eval_tc_kernel.cuh"
+#include "loo.cuh"
 #include "newton.cuh"
 #include "predictive.cuh"
 #include "sampler.cuh"
@@ -1201,6 +1202,244 @@ extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int
     totals->elpd_waic = tot[2];
     totals->se_elpd_waic = tot[3];
   }
+  return LRB_OK;
+}
+
+// ============================================================ PSIS-LOO / pointwise log-likelihood
+namespace {
+
+using LoglikFn = void (*)(const LoglikArgs);
+
+template <typename T>
+LoglikFn pick_loglik(int P, size_t& smem) {
+  switch (P) {
+    case 8: smem = predictive_smem<T, 8>(); return loglik_kernel<T, 8>;
+    case 16: smem = predictive_smem<T, 16>(); return loglik_kernel<T, 16>;
+    case 32: smem = predictive_smem<T, 32>(); return loglik_kernel<T, 32>;
+    case 64: smem = predictive_smem<T, 64>(); return loglik_kernel<T, 64>;
+    case 128: smem = predictive_smem<T, 128>(); return loglik_kernel<T, 128>;
+    case 256: smem = predictive_smem<T, 256>(); return loglik_kernel<T, 256>;
+  }
+  return nullptr;
+}
+
+// Stage 1 for one handle and one set of draws: the uploaded draws and the kernel's launch shape.
+struct Loglik {
+  DevTmp dB;
+  LoglikFn fn = nullptr;
+  size_t smem = 0;
+  int occ = 0;
+  long long S = 0, Spad = 0;
+};
+
+int loglik_prepare(lrb_handle* h, const double* draws, long long S, Loglik& g) {
+  const bool fp32 = h->mode == LRB_MODE_FP32;
+  g.fn = fp32 ? pick_loglik<float>(h->P, g.smem) : pick_loglik<double>(h->P, g.smem);
+  if (!g.fn) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", h->P);
+  CK(h, cudaFuncSetAttribute((const void*)g.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
+  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g.occ, g.fn, kBlock, g.smem));
+  if (g.occ < 1) return fail(h, LRB_E_CUDA, "log-likelihood kernel does not fit an SM");
+  g.S = S;
+  g.Spad = (S + kPredDraws - 1) / kPredDraws * kPredDraws;
+  CK(h, g.dB.alloc((size_t)h->P * g.Spad * (fp32 ? 4 : 8)));
+  return fp32 ? upload_draws<float>(h, g.dB.p, draws, S, g.Spad) : upload_draws<double>(h, g.dB.p, draws, S, g.Spad);
+}
+
+// L[i][s] (row stride S) for the bound rows [row0, row0 + rows)
+int loglik_launch(lrb_handle* h, const Loglik& g, long long row0, long long rows, double* L) {
+  const size_t es = h->mode == LRB_MODE_FP32 ? 4 : 8;
+  LoglikArgs a{};
+  a.X = static_cast<const char*>(h->X) + (size_t)row0 * h->P * es;
+  a.y = h->y + row0;
+  a.n = rows;
+  a.B = g.dB.p; a.S = g.S; a.Spad = g.Spad;
+  a.L = L; a.ld = g.S;
+  const long long ntiles = (rows + kPredRows - 1) / kPredRows;
+  const long long ngroups = (g.Spad / kPredDraws + kLoglikGroup - 1) / kLoglikGroup;
+  const int grid = (int)std::min<long long>((long long)h->sms * g.occ, ntiles * ngroups);
+  g.fn<<<grid, kBlock, g.smem, h->stream>>>(a);
+  CK(h, cudaGetLastError());
+  h->kernel_launches++;
+  return LRB_OK;
+}
+
+// Rows of L per chunk: a multiple of 64 whose L fits the scratch budget (at least 64 rows).
+// LRB_LOO_CHUNK_MB overrides the budget, to measure what keeping a chunk in L2 is worth.
+long long loo_chunk_rows(long long n, long long S) {
+  long long budget = 64ll << 20;
+  if (const char* e = getenv("LRB_LOO_CHUNK_MB")) budget = std::max(1ll, atoll(e)) << 20;
+  long long R = budget / (S * (long long)sizeof(double)) / kPredRows * kPredRows;
+  R = std::max<long long>(R, kPredRows);
+  return std::min<long long>(R, (n + kPredRows - 1) / kPredRows * kPredRows);
+}
+
+int check_single_gpu(lrb_handle* h, const char* what) {
+  if (h->world > 1)
+    return fail(h, LRB_E_UNSUPPORTED, "%s works on single-GPU handles only: this handle is rank %d of a row-sharded "
+                "group of %d, and its per-shard totals would need a collective", what, h->rank, h->world);
+  return LRB_OK;
+}
+
+}  // namespace
+
+extern "C" int lrb_loglik(lrb_handle* h, const double* draws, int64_t S, int64_t row0, int64_t nrows, int location,
+                          double* out) {
+  if (!h) return fail(nullptr, LRB_E_BAD_ARG, "handle is NULL");
+  if (!h->bound) return fail(h, LRB_E_STATE, "lrb_loglik before lrb_bind_data / lrb_gen_synthetic");
+  if (!draws || !out || S < 1) return fail(h, LRB_E_BAD_ARG, "draws or out is NULL, or S < 1 (S=%lld)", (long long)S);
+  if (S > kLooMaxDraws) return fail(h, LRB_E_BAD_ARG, "S=%lld draws exceeds 2^21", (long long)S);
+  if (row0 < 0 || nrows < 1 || row0 + nrows > h->n)
+    return fail(h, LRB_E_BAD_ARG, "rows [%lld, %lld) outside the %lld bound rows", (long long)row0,
+                (long long)(row0 + nrows), h->n);
+  if (location != LRB_HOST && location != LRB_DEVICE) return fail(h, LRB_E_BAD_ARG, "bad location %d", location);
+  if (int rc = check_single_gpu(h, "lrb_loglik")) return rc;
+  if (use_device(h)) return LRB_E_CUDA;
+  Loglik g;
+  if (int rc = loglik_prepare(h, draws, S, g)) return rc;
+  if (location == LRB_DEVICE) {
+    if (int rc = loglik_launch(h, g, row0, nrows, out)) return rc;
+  } else {   // chunk by chunk through a bounded device buffer
+    const long long R = loo_chunk_rows(nrows, S);
+    DevTmp L;
+    CK(h, L.alloc((size_t)R * S * sizeof(double)));
+    for (long long c0 = 0; c0 < nrows; c0 += R) {
+      const long long rows = std::min(R, (long long)nrows - c0);
+      if (int rc = loglik_launch(h, g, row0 + c0, rows, L.as<double>())) return rc;
+      CK(h, cudaMemcpyAsync(out + (size_t)c0 * S, L.p, (size_t)rows * S * sizeof(double), cudaMemcpyDeviceToHost,
+                            h->stream));
+    }
+  }
+  CK(h, cudaStreamSynchronize(h->stream));   // the temporaries die with this scope
+  return LRB_OK;
+}
+
+extern "C" int lrb_loo(lrb_handle* h, const double* draws, int64_t S, int location, double* elpd_loo, double* p_loo,
+                       double* pareto_k, lrb_loo_totals* totals) {
+  if (!h) return fail(nullptr, LRB_E_BAD_ARG, "handle is NULL");
+  if (!h->bound) return fail(h, LRB_E_STATE, "lrb_loo before lrb_bind_data / lrb_gen_synthetic");
+  if (!draws || S < 1) return fail(h, LRB_E_BAD_ARG, "draws is NULL or S < 1 (S=%lld)", (long long)S);
+  if (S > kLooMaxDraws)
+    return fail(h, LRB_E_BAD_ARG, "S=%lld draws exceeds 2^21: PSIS needs a row's S log-likelihoods at once, and 64 "
+                "rows of them (the smallest chunk) would exceed 1 GB of scratch", (long long)S);
+  if (location != LRB_HOST && location != LRB_DEVICE) return fail(h, LRB_E_BAD_ARG, "bad location %d", location);
+  if (int rc = check_single_gpu(h, "lrb_loo")) return rc;
+  if (use_device(h)) return LRB_E_CUDA;
+  const bool stage2 = !getenv("LRB_LOO_STAGE1_ONLY");   // timing of stage 1 alone (header, tools/loo_bench.py)
+  Loglik g;
+  if (int rc = loglik_prepare(h, draws, S, g)) return rc;
+  const long long n = h->n, M = psis_tail_len(S);
+  const int stage = S <= kLooRowSmem ? 1 : 0;
+  const size_t smem = psis_smem(S, M, stage);
+  CK(h, cudaFuncSetAttribute((const void*)psis_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, psis_kernel, kBlock, smem));
+  if (occ < 1) return fail(h, LRB_E_CUDA, "PSIS kernel does not fit an SM");
+
+  const long long R = loo_chunk_rows(n, S);
+  const long long ntiles = (n + kPredRows - 1) / kPredRows;
+  DevTmp L, rowbuf, work;
+  CK(h, L.alloc((size_t)R * S * sizeof(double)));
+  CK(h, rowbuf.alloc((size_t)3 * R * sizeof(double)));
+  CK(h, work.alloc(((size_t)ntiles * kLooPartial + 8) * sizeof(double)));
+  double* re = rowbuf.as<double>();
+  double *rp = re + R, *rk = rp + R;
+  double* partials = work.as<double>();
+  double* dtot = partials + (size_t)ntiles * kLooPartial;
+  double* user[3] = {elpd_loo, p_loo, pareto_k};
+  double* chunk[3] = {re, rp, rk};
+  const cudaMemcpyKind kind = location == LRB_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+  const double kthr = loo_k_threshold(S);
+  for (long long c0 = 0; c0 < n; c0 += R) {
+    const long long rows = std::min(R, n - c0);
+    if (int rc = loglik_launch(h, g, c0, rows, L.as<double>())) return rc;
+    if (!stage2) continue;
+    PsisArgs a{};
+    a.L = L.as<double>(); a.rows = rows; a.S = S; a.M = M; a.stage = stage;
+    a.elpd = re; a.p_loo = rp; a.pareto_k = rk;
+    psis_kernel<<<(int)std::min<long long>((long long)h->sms * occ, rows), kBlock, smem, h->stream>>>(a);
+    CK(h, cudaGetLastError());
+    const long long ct = (rows + kPredRows - 1) / kPredRows;
+    loo_tile_kernel<<<(int)((ct + kBlock - 1) / kBlock), kBlock, 0, h->stream>>>(re, rp, rk, rows, kthr,
+                                                                               partials + (c0 / kPredRows) * kLooPartial);
+    CK(h, cudaGetLastError());
+    h->kernel_launches += 2;
+    for (int k = 0; k < 3; ++k)
+      if (user[k]) CK(h, cudaMemcpyAsync(user[k] + c0, chunk[k], (size_t)rows * sizeof(double), kind, h->stream));
+  }
+  double tot[7];
+  for (double& t : tot) t = NAN;
+  if (!stage2)   // stage 1 was timed alone: no result exists, so every output reads NaN
+    for (int k = 0; k < 3; ++k) {
+      if (!user[k]) continue;
+      if (location == LRB_DEVICE) CK(h, cudaMemsetAsync(user[k], 0xff, (size_t)n * sizeof(double), h->stream));
+      else std::fill(user[k], user[k] + n, (double)NAN);
+    }
+  if (stage2) {
+    loo_totals_kernel<<<1, kBlock, 0, h->stream>>>(partials, ntiles, dtot);
+    CK(h, cudaGetLastError());
+    h->kernel_launches++;
+    CK(h, cudaMemcpyAsync(tot, dtot, sizeof tot, cudaMemcpyDeviceToHost, h->stream));
+  }
+  CK(h, cudaStreamSynchronize(h->stream));   // the temporaries die with this scope
+  if (totals) {
+    totals->n = n;
+    totals->draws = S;
+    totals->elpd_loo = tot[1];
+    totals->se_elpd_loo = tot[2];
+    totals->p_loo = tot[3];
+    totals->se_p_loo = tot[4];
+    totals->looic = -2.0 * tot[1];
+    totals->k_threshold = kthr;
+    totals->k_max = tot[5];
+    totals->n_k_high = stage2 ? (int64_t)tot[6] : -1;
+  }
+  return LRB_OK;
+}
+
+extern "C" int lrb_debug_psis(const double* log_ratios, int64_t S, double* log_weights, double* khat) {
+  if (!log_ratios || !log_weights || !khat || S < 1) return fail(nullptr, LRB_E_BAD_ARG, "bad arguments");
+  const double* r = log_ratios;
+  double rmax = r[0];
+  for (int64_t s = 1; s < S; ++s) rmax = nan_max(rmax, r[s]);
+  std::vector<double> lw(S);
+  for (int64_t s = 0; s < S; ++s) lw[s] = r[s] - rmax;
+  double k = INFINITY;
+  const int64_t M = psis_tail_len(S);
+  if (M >= 5) {
+    std::vector<int64_t> order(S);
+    for (int64_t s = 0; s < S; ++s) order[s] = s;
+    std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return lw[a] < lw[b]; });
+    const double tmin = lw[order[S - M]], tmax = lw[order[S - 1]];
+    if (std::fabs(tmax - tmin) >= 2.220446049250313e-16 / 100.0) {
+      const double cutoff = lw[order[S - M - 1]], ec = std::exp(cutoff);
+      std::vector<double> x(M);
+      for (int64_t j = 0; j < M; ++j) x[j] = std::exp(lw[order[S - M + j]]) - ec;
+      const int mg = gpd_grid_len(M);
+      const double xmax = x[M - 1], xstar = x[(int64_t)std::floor(M / 4.0 + 0.5) - 1];
+      std::vector<double> th(mg), lt(mg);
+      double lmx = -INFINITY;
+      for (int j = 0; j < mg; ++j) {
+        th[j] = gpd_theta(j + 1, mg, xmax, xstar);
+        double sk = 0.0;
+        for (int64_t t = 0; t < M; ++t) sk += std::log1p(-th[j] * x[t]);
+        lt[j] = gpd_ltheta(th[j], sk / (double)M, M);
+        lmx = nan_max(lmx, lt[j]);
+      }
+      double sw = 0.0;
+      for (int j = 0; j < mg; ++j) sw += std::exp(lt[j] - lmx);
+      const double lse = lmx + std::log(sw);
+      double theta = 0.0;
+      for (int j = 0; j < mg; ++j) theta += th[j] * std::exp(lt[j] - lse);
+      double sk = 0.0;
+      for (int64_t t = 0; t < M; ++t) sk += std::log1p(-theta * x[t]);
+      const double kraw = sk / (double)M, sigma = -kraw / theta;
+      k = gpd_wip(kraw, M);
+      if (std::isfinite(k))
+        for (int64_t j = 0; j < M; ++j) lw[order[S - M + j]] = psis_smoothed(k, sigma, psis_quantile(j + 1, M), ec);
+    }
+  }
+  for (int64_t s = 0; s < S; ++s) log_weights[s] = (lw[s] > 0.0 ? 0.0 : lw[s]) + rmax;
+  *khat = k;
   return LRB_OK;
 }
 

@@ -20,6 +20,11 @@ Beyond the reference (which stops at the samples), over S posterior draws on the
                     training rows, or the held-out lppd on a Problem bound to test rows
     waic_from_pointwise  the same totals from per-row lppd / p_waic arrays, e.g. of several Problems
     predict_proba   posterior mean and sd of P(y = 1 | x) for unlabelled rows
+and PSIS-LOO (lrb_loo: Pareto-smoothed importance-sampling leave-one-out, R's loo::loo()):
+    loo             elpd_loo, p_loo, looic and their SEs, with the Pareto k-hat diagnostic (k_max,
+                    n_k_high) of the rows bound to a Problem
+    loo_from_pointwise  the same totals from per-row elpd_loo / p_loo / pareto_k, e.g. of several Problems
+    loo_compare     elpd difference of two models on the same rows and its SE (loo::loo_compare)
 """
 from __future__ import annotations
 
@@ -140,6 +145,48 @@ def waic_from_pointwise(lppd, p_waic, draws):
     return {"elpd_waic": float(elpd.sum()), "p_waic": float(p_waic.sum()), "lppd": float(lppd.sum()),
             "se_elpd_waic": float(np.sqrt(n * elpd.var(ddof=1))) if n > 1 else float("nan"),
             "n": n, "draws": int(draws)}
+
+
+_LOO_KEYS = ("elpd_loo", "se_elpd_loo", "p_loo", "se_p_loo", "looic", "se_looic", "k_threshold", "k_max",
+             "n_k_high", "n", "draws")
+
+
+def loo(problem, draws):
+    """PSIS-LOO of the rows bound to `problem` over posterior draws (S, p) or (C, iters, p), as
+    R's loo package reports it (r_eff = 1): {elpd_loo, se_elpd_loo, p_loo, se_p_loo, looic,
+    se_looic, k_threshold, k_max, n_k_high, n, draws}. Rows with pareto_k > k_threshold (n_k_high of
+    them) have unreliable elpd_loo terms. Nothing per row leaves the device."""
+    t = problem.loo(draws, pointwise=False)
+    return {k: t[k] for k in _LOO_KEYS}
+
+
+def _se(v):
+    n = v.shape[0]
+    return float(np.sqrt(n * v.var(ddof=1))) if n > 1 else float("nan")
+
+
+def loo_from_pointwise(elpd_loo, p_loo, pareto_k, draws):
+    """The totals of `loo` from per-row arrays (loo(...)["pointwise"]), e.g. concatenated over
+    Problems holding parts of one data set; `draws` is S."""
+    e = np.asarray(elpd_loo, dtype=np.float64)
+    p = np.asarray(p_loo, dtype=np.float64)
+    k = np.asarray(pareto_k, dtype=np.float64)
+    thr = min(1.0 - 1.0 / np.log10(draws), 0.7) if draws > 1 else -np.inf
+    return {"elpd_loo": float(e.sum()), "se_elpd_loo": _se(e), "p_loo": float(p.sum()), "se_p_loo": _se(p),
+            "looic": -2.0 * float(e.sum()), "se_looic": 2.0 * _se(e), "k_threshold": float(thr),
+            "k_max": float(k.max()), "n_k_high": int(np.sum(k > thr)), "n": e.shape[0], "draws": int(draws)}
+
+
+def loo_compare(elpd_a, elpd_b):
+    """Model comparison on the same rows from pointwise elpd_loo (loo::loo_compare for two models):
+    elpd_diff = sum(elpd_a - elpd_b) (positive: model a predicts better) and
+    se_diff = sqrt(n var(elpd_a - elpd_b)) (ddof 1)."""
+    a = np.asarray(elpd_a, dtype=np.float64)
+    b = np.asarray(elpd_b, dtype=np.float64)
+    if a.shape != b.shape or a.ndim != 1:
+        raise ValueError(f"pointwise elpd of both models must be 1-D over the same rows, got {a.shape} and {b.shape}")
+    d = a - b
+    return {"elpd_diff": float(d.sum()), "se_diff": _se(d)}
 
 
 def predict_proba(X_new, draws, mode="fp64", device=0):
