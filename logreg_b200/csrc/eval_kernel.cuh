@@ -139,48 +139,59 @@ __device__ __forceinline__ double row_terms(double eta, bool y1, double& r) {
   return fmin(z, 0.0) - log1p(e);
 }
 
-template <typename T, int P, bool GRAD>
-__global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
+// One warp's row batch in the SIMT evaluation kernels (eval_kernel, eval_persist_kernel,
+// eval_mc_kernel): the tiling, this lane's place in it, and the per-batch arithmetic (steps 1-4
+// above).  The kernels own only which batches a warp takes and where the sums go.
+template <typename T, int P>
+struct BatchTile {
   using C = Chunk<T>;
   using vec = typename C::vec;
   using A = typename C::acc_t;
-  constexpr int V = C::V;
-  constexpr int CPR = P / V;                // 16-byte chunks per row
-  constexpr int L = CPR < 32 ? CPR : 32;    // lanes sharing a row inside one slab
-  constexpr int SPR = CPR / L;              // slabs per row (>1 when a row exceeds 512 B)
-  constexpr int G = 32 / L;                 // rows per slab (SPR == 1)
-  constexpr int S = 16;                     // slabs per batch
-  constexpr int SG = S / SPR;               // row groups per batch
-  constexpr int RB = SG * G;                // rows per batch
-  constexpr int LOG_L = ilog2(L), LOG_SG = ilog2(SG);
-  constexpr int NH = LOG_L < LOG_SG ? LOG_L : LOG_SG;  // halving rounds
-  constexpr int M = SG >> NH;               // etas a lane owns per batch
+  static constexpr int V = C::V;
+  static constexpr int CPR = P / V;                // 16-byte chunks per row
+  static constexpr int L = CPR < 32 ? CPR : 32;    // lanes sharing a row inside one slab
+  static constexpr int SPR = CPR / L;              // slabs per row (>1 when a row exceeds 512 B)
+  static constexpr int G = 32 / L;                 // rows per slab (SPR == 1)
+  static constexpr int S = 16;                     // slabs per batch
+  static constexpr int SG = S / SPR;               // row groups per batch
+  static constexpr int RB = SG * G;                // rows per batch
+  static constexpr int LOG_L = ilog2(L), LOG_SG = ilog2(SG);
+  static constexpr int NH = LOG_L < LOG_SG ? LOG_L : LOG_SG;  // halving rounds
+  static constexpr int M = SG >> NH;               // etas a lane owns per batch
   static_assert(S % SPR == 0 && SG >= 1, "row too wide for the batch");
   static_assert((1 << LOG_L) == L && (1 << LOG_SG) == SG, "power-of-two tiling");
 
-  __shared__ double red[kWarps][P + 1];
-  __shared__ double redll[kWarps];
-  __shared__ double tot[P + 1];
-  __shared__ double scratch[kWarps];
-  __shared__ unsigned int s_ticket;
+  // this lane's slice of a coefficient vector, columns (sl*L + t_in_row)*V .. +V, as hi + lo
+  // (lo is exactly 0 in FP64 mode)
+  struct Coef {
+    A hi[SPR][V];
+    float lo[SPR][V];
+  };
+  // labels and validity of the M rows this lane owns in a batch
+  struct Rows {
+    bool y1[M], valid[M];
+  };
 
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int t_in_row = lane & (L - 1);      // which chunk of the row segment
-  const int g_in_slab = lane >> LOG_L;      // which row of the slab
-  const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
-  const long long n = a.n;
-  const long long total_chunks = n * CPR;
-  const long long nbatch = (n + RB - 1) / RB;
-  const long long nwarps = (long long)gridDim.x * kWarps;
-  const long long bt0 = (long long)blockIdx.x * kWarps + warp;
+  long long n;              // rows of X
+  long long total_chunks;   // 16-byte chunks of X; formed here, once: formed in load, it changed how the
+                            // compiler unrolls the drive kernel's finish step
+  long long nbatch;         // batches of X, the last one possibly partial
+  int lane;
+  int t_in_row;    // which chunk of the row segment
+  int g_in_slab;   // which row of the slab
+  int khigh;       // rows this lane owns after the exchange: k = j + khigh, row = row0 + k*G + g_in_slab
+  bool owner;
 
-  // Programmatic dependent launch: this grid may start while the previous evaluation's last
-  // CTA is still reducing / running the sampler update.  X never changes, so the first batch
-  // is fetched BEFORE waiting for the previous grid (hides launch latency and the DRAM ramp);
-  // everything that depends on it (beta, the pause flag, the partials buffer) comes after.
-  EV_STAMP(0);
-  vec v[S];
-  auto load_batch = [&](long long bt) {
+  __device__ __forceinline__ BatchTile(long long n_, int lane_)
+      : n(n_), total_chunks(n_ * CPR), nbatch((n_ + RB - 1) / RB), lane(lane_), t_in_row(lane_ & (L - 1)),
+        g_in_slab(lane_ >> LOG_L), khigh(0) {
+#pragma unroll
+    for (int b = 0; b < NH; ++b) khigh += ((t_in_row >> b) & 1) * (SG >> (b + 1));
+    owner = (t_in_row >> NH) == 0;
+  }
+
+  // The S slabs of batch bt; chunks past the end of X read as zero.
+  __device__ __forceinline__ void load(vec (&v)[S], const vec* __restrict__ Xv, long long bt) const {
     const long long chunk0 = bt * (S * 32) + lane;
     if (bt * RB + RB <= n) {
 #pragma unroll
@@ -192,52 +203,36 @@ __global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
         v[s] = c < total_chunks ? ldg_stream(Xv + c) : zero_vec((vec*)nullptr);
       }
     }
-  };
-  if (bt0 < nbatch) load_batch(bt0);
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  EV_STAMP(1);
+  }
 
-  // A paused sampler makes surplus graph nodes no-ops (every CTA sees the same phase:
-  // the last CTA only changes it after all CTAs have taken their ticket).
-  if (a.fin.state != nullptr && __ldcg(&a.fin.state->phase) == PH_PAUSED) return;
+  // Read through L2: in the fused kernels the previous evaluation's last CTA wrote beta.
+  __device__ __forceinline__ void load_coef(Coef& cf, const double* beta, int p) const {
+#pragma unroll
+    for (int sl = 0; sl < SPR; ++sl)
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        const int col = (sl * L + t_in_row) * V + i;
+        const double x = col < p ? __ldcg(beta + col) : 0.0;
+        cf.hi[sl][i] = (A)x;
+        cf.lo[sl][i] = (float)(x - (double)cf.hi[sl][i]);
+      }
+  }
 
-  // this lane's slice of beta (read through L2: the previous grid's last CTA wrote it) (columns (sl*L + t_in_row)*V .. +V)
-  A bh[SPR][V];
-  float bl[SPR][V];
-#pragma unroll
-  for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-      const int col = (sl * L + t_in_row) * V + i;
-      const double b = col < a.fin.p ? __ldcg(a.fin.beta + col) : 0.0;
-      bh[sl][i] = (A)b;
-      bl[sl][i] = (float)(b - (double)bh[sl][i]);   // exactly 0 in FP64 mode
-    }
-
-  // rows this lane will own after the exchange: k = j + khigh, row = row0 + k*G + g
-  int khigh = 0;
-#pragma unroll
-  for (int b = 0; b < NH; ++b) khigh += ((t_in_row >> b) & 1) * (SG >> (b + 1));
-  const bool owner = (t_in_row >> NH) == 0;
-
-  double acc[SPR][V];
-#pragma unroll
-  for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-    for (int i = 0; i < V; ++i) acc[sl][i] = 0.0;
-  double ll_acc = 0.0;
-
-  for (long long bt = bt0; bt < nbatch; bt += nwarps) {
+  __device__ __forceinline__ void load_rows(Rows& rw, const uint8_t* y, long long bt) const {
     const long long row0 = bt * RB;
-    if (bt != bt0) load_batch(bt);
-    bool y1[M], valid[M];
 #pragma unroll
     for (int j = 0; j < M; ++j) {
       const long long row = row0 + (long long)(j + khigh) * G + g_in_slab;
-      valid[j] = owner && row < n;
-      y1[j] = valid[j] ? (a.y[row] != 0) : false;
+      rw.valid[j] = owner && row < n;
+      rw.y1[j] = rw.valid[j] ? (y[row] != 0) : false;
     }
+  }
 
+  // One batch at one coefficient vector: the rows' log-likelihood terms into ll, and with GRAD
+  // this lane's gradient columns into acc.
+  template <bool GRAD>
+  __device__ __forceinline__ void accumulate(const vec (&v)[S], const Rows& rw, const Coef& cf, double& ll,
+                                             double (&acc)[SPR][V]) const {
     // 1. partial dot products, combined over the slabs of a row
     A q[SG];
 #pragma unroll
@@ -246,13 +241,13 @@ __global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
 #pragma unroll
       for (int sl = 0; sl < SPR; ++sl)
 #pragma unroll
-        for (int i = 0; i < V; ++i) s_hi = fma(elem(v[k * SPR + sl], i), bh[sl][i], s_hi);
+        for (int i = 0; i < V; ++i) s_hi = fma(elem(v[k * SPR + sl], i), cf.hi[sl][i], s_hi);
       if constexpr (sizeof(T) == 4) {
         float s_lo = 0.f;
 #pragma unroll
         for (int sl = 0; sl < SPR; ++sl)
 #pragma unroll
-          for (int i = 0; i < V; ++i) s_lo = fmaf((float)elem(v[k * SPR + sl], i), bl[sl][i], s_lo);
+          for (int i = 0; i < V; ++i) s_lo = fmaf((float)elem(v[k * SPR + sl], i), cf.lo[sl][i], s_lo);
         s_hi += (A)s_lo;
       }
       q[k] = s_hi;
@@ -265,9 +260,9 @@ __global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
 #pragma unroll
     for (int j = 0; j < M; ++j) {
       A rr;
-      const A lt = row_terms(q[j], y1[j], rr);
+      const A lt = row_terms(q[j], rw.y1[j], rr);
       r[j] = rr;
-      if (valid[j]) ll_acc += (double)lt;
+      if (rw.valid[j]) ll += (double)lt;
     }
 
     // 4. gradient: g[cols of this lane] += r(row) * x
@@ -296,11 +291,8 @@ __global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
     }
   }
 
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // streaming done: let the next grid in
-  EV_STAMP(2);
-
-  // ---- CTA reduction
-  if constexpr (GRAD) {
+  // The warp's gradient sums: acc over the lanes of equal t_in_row, column c to dst[c].
+  __device__ __forceinline__ void store_grad(const double (&acc)[SPR][V], double* dst) const {
 #pragma unroll
     for (int sl = 0; sl < SPR; ++sl)
 #pragma unroll
@@ -308,9 +300,60 @@ __global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
         double x = acc[sl][i];
 #pragma unroll
         for (int o = L; o < 32; o <<= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-        if (lane < L) red[warp][(sl * L + lane) * V + i] = x;
+        if (lane < L) dst[(sl * L + lane) * V + i] = x;
       }
   }
+};
+
+template <typename T, int P, bool GRAD>
+__global__ void __launch_bounds__(kBlock, 2) eval_kernel(const EvalArgs a) {
+  using Tile = BatchTile<T, P>;
+  using vec = typename Tile::vec;
+
+  __shared__ double red[kWarps][P + 1];
+  __shared__ double redll[kWarps];
+  __shared__ double tot[P + 1];
+  __shared__ double scratch[kWarps];
+  __shared__ unsigned int s_ticket;
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const Tile tl(a.n, lane);
+  const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
+  const long long nbatch = tl.nbatch;
+  const long long nwarps = (long long)gridDim.x * kWarps;
+  const long long bt0 = (long long)blockIdx.x * kWarps + warp;
+
+  // Programmatic dependent launch: this grid may start while the previous evaluation's last
+  // CTA is still reducing / running the sampler update.  X never changes, so the first batch
+  // is fetched BEFORE waiting for the previous grid (hides launch latency and the DRAM ramp);
+  // everything that depends on it (beta, the pause flag, the partials buffer) comes after.
+  EV_STAMP(0);
+  vec v[Tile::S];
+  if (bt0 < nbatch) tl.load(v, Xv, bt0);
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  EV_STAMP(1);
+
+  // A paused sampler makes surplus graph nodes no-ops (every CTA sees the same phase:
+  // the last CTA only changes it after all CTAs have taken their ticket).
+  if (a.fin.state != nullptr && __ldcg(&a.fin.state->phase) == PH_PAUSED) return;
+
+  typename Tile::Coef cf;
+  tl.load_coef(cf, a.fin.beta, a.fin.p);
+  double acc[Tile::SPR][Tile::V] = {};
+  double ll_acc = 0.0;
+
+  for (long long bt = bt0; bt < nbatch; bt += nwarps) {
+    if (bt != bt0) tl.load(v, Xv, bt);
+    typename Tile::Rows rw;
+    tl.load_rows(rw, a.y, bt);
+    tl.template accumulate<GRAD>(v, rw, cf, ll_acc, acc);
+  }
+
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // streaming done: let the next grid in
+  EV_STAMP(2);
+
+  // ---- CTA reduction
+  if constexpr (GRAD) tl.store_grad(acc, red[warp]);
   ll_acc = warp_sum(ll_acc);
   if (lane == 0) redll[warp] = ll_acc;
   __syncthreads();

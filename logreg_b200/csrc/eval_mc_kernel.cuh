@@ -4,8 +4,8 @@
 // above the chain-count threshold the tcgen05 kernel (eval_tc_kernel.cuh) takes
 // over, where eta = X B' and G = R' X become tensor-core contractions.
 //
-// Same arithmetic per chain as eval_kernel (see eval_kernel.cuh for the lane
-// mapping); the finish step runs in a separate launch with one CTA per chain.
+// Each chain's batch goes through BatchTile (eval_kernel.cuh), as in the single-chain kernels;
+// the finish step runs in a separate launch with one CTA per chain.
 #pragma once
 #include "eval_kernel.cuh"
 
@@ -29,20 +29,8 @@ struct EvalMcArgs {
 
 template <typename T, int P, int NC>
 __global__ void __launch_bounds__(kBlock, 1) eval_mc_kernel(const EvalMcArgs a) {
-  using C = Chunk<T>;
-  using vec = typename C::vec;
-  using A = typename C::acc_t;
-  constexpr int V = C::V;
-  constexpr int CPR = P / V;
-  constexpr int L = CPR < 32 ? CPR : 32;
-  constexpr int SPR = CPR / L;
-  constexpr int G = 32 / L;
-  constexpr int S = 16;
-  constexpr int SG = S / SPR;
-  constexpr int RB = SG * G;
-  constexpr int LOG_L = ilog2(L), LOG_SG = ilog2(SG);
-  constexpr int NH = LOG_L < LOG_SG ? LOG_L : LOG_SG;
-  constexpr int M = SG >> NH;
+  using Tile = BatchTile<T, P>;
+  using vec = typename Tile::vec;
 
   __shared__ double red[kWarps][P];
   __shared__ double redll[kWarps];
@@ -51,134 +39,33 @@ __global__ void __launch_bounds__(kBlock, 1) eval_mc_kernel(const EvalMcArgs a) 
   if (a.states != nullptr && a.states[a.chain0].phase == PH_PAUSED) return;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int t_in_row = lane & (L - 1);
-  const int g_in_slab = lane >> LOG_L;
+  const Tile tl(a.n, lane);
   const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
-  const long long n = a.n;
-  const long long total_chunks = n * CPR;
-  const long long nbatch = (n + RB - 1) / RB;
+  const long long nbatch = tl.nbatch;
 
-  A bh[NC][SPR][V];
-  float bl[NC][SPR][V];
+  typename Tile::Coef cf[NC];
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int cc = c < a.nc_active ? c : 0;   // surplus slots recompute chain0's first chain (discarded)
-    const double* beta = a.beta_base + (long long)(a.chain0 + cc) * a.beta_stride;
-#pragma unroll
-    for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int col = (sl * L + t_in_row) * V + i;
-        const double b = col < a.p ? beta[col] : 0.0;
-        bh[c][sl][i] = (A)b;
-        bl[c][sl][i] = (float)(b - (double)bh[c][sl][i]);
-      }
+    tl.load_coef(cf[c], a.beta_base + (long long)(a.chain0 + cc) * a.beta_stride, a.p);
   }
-
-  int khigh = 0;
-#pragma unroll
-  for (int b = 0; b < NH; ++b) khigh += ((t_in_row >> b) & 1) * (SG >> (b + 1));
-  const bool owner = (t_in_row >> NH) == 0;
-
-  double acc[NC][SPR][V];
-  double ll_acc[NC];
-#pragma unroll
-  for (int c = 0; c < NC; ++c) {
-    ll_acc[c] = 0.0;
-#pragma unroll
-    for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-      for (int i = 0; i < V; ++i) acc[c][sl][i] = 0.0;
-  }
+  double acc[NC][Tile::SPR][Tile::V] = {};
+  double ll_acc[NC] = {};
 
   const long long nwarps = (long long)gridDim.x * kWarps;
   for (long long bt = (long long)blockIdx.x * kWarps + warp; bt < nbatch; bt += nwarps) {
-    const long long chunk0 = bt * (S * 32) + lane;
-    const long long row0 = bt * RB;
-    vec v[S];
-    if (row0 + RB <= n) {
+    vec v[Tile::S];
+    tl.load(v, Xv, bt);
+    typename Tile::Rows rw;
+    tl.load_rows(rw, a.y, bt);
 #pragma unroll
-      for (int s = 0; s < S; ++s) v[s] = ldg_stream(Xv + chunk0 + s * 32);
-    } else {
-#pragma unroll
-      for (int s = 0; s < S; ++s) {
-        const long long c = chunk0 + s * 32;
-        v[s] = c < total_chunks ? ldg_stream(Xv + c) : zero_vec((vec*)nullptr);
-      }
-    }
-    bool y1[M], valid[M];
-#pragma unroll
-    for (int j = 0; j < M; ++j) {
-      const long long row = row0 + (long long)(j + khigh) * G + g_in_slab;
-      valid[j] = owner && row < n;
-      y1[j] = valid[j] ? (a.y[row] != 0) : false;
-    }
-
-#pragma unroll
-    for (int c = 0; c < NC; ++c) {
-      A q[SG];
-#pragma unroll
-      for (int k = 0; k < SG; ++k) {
-        A s_hi = (A)0;
-#pragma unroll
-        for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-          for (int i = 0; i < V; ++i) s_hi = fma(elem(v[k * SPR + sl], i), bh[c][sl][i], s_hi);
-        if constexpr (sizeof(T) == 4) {
-          float s_lo = 0.f;
-#pragma unroll
-          for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-            for (int i = 0; i < V; ++i) s_lo = fmaf((float)elem(v[k * SPR + sl], i), bl[c][sl][i], s_lo);
-          s_hi += (A)s_lo;
-        }
-        q[k] = s_hi;
-      }
-      reduce_rows<SG, 0, LOG_L>(q, lane);
-      A r[M];
-#pragma unroll
-      for (int j = 0; j < M; ++j) {
-        A rr;
-        const A lt = row_terms(q[j], y1[j], rr);
-        r[j] = rr;
-        if (valid[j]) ll_acc[c] += (double)lt;
-      }
-      A gb[SPR][V];
-#pragma unroll
-      for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-        for (int i = 0; i < V; ++i) gb[sl][i] = (A)0;
-#pragma unroll
-      for (int k = 0; k < SG; ++k) {
-        const int j = k & (M - 1);
-        int tsrc = 0;
-#pragma unroll
-        for (int b = 0; b < NH; ++b) tsrc |= ((k >> (LOG_SG - 1 - b)) & 1) << b;
-        const A rr = __shfl_sync(0xffffffffu, r[j], (lane & ~(L - 1)) | tsrc);
-#pragma unroll
-        for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-          for (int i = 0; i < V; ++i) gb[sl][i] = fma(rr, (A)elem(v[k * SPR + sl], i), gb[sl][i]);
-      }
-#pragma unroll
-      for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-        for (int i = 0; i < V; ++i) acc[c][sl][i] += (double)gb[sl][i];
-    }
+    for (int c = 0; c < NC; ++c) tl.template accumulate<true>(v, rw, cf[c], ll_acc[c], acc[c]);
   }
 
   // ---- CTA reduction, one chain at a time through the same scratch
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
-#pragma unroll
-    for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        double x = acc[c][sl][i];
-#pragma unroll
-        for (int o = L; o < 32; o <<= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-        if (lane < L) red[warp][(sl * L + lane) * V + i] = x;
-      }
+    tl.store_grad(acc[c], red[warp]);
     const double lw = warp_sum(ll_acc[c]);
     if (lane == 0) redll[warp] = lw;
     __syncthreads();

@@ -2,9 +2,10 @@
 // launch runs a whole sequence of evaluations (BASELINE.json north_star (c): "CUDA Graphs or a
 // persistent kernel so no per-iteration host round-trip remains").
 //
-// Same arithmetic per row batch as eval_kernel.cuh (see there for the lane mapping and the
-// reference lines: ll Python/fit-numpy.py:23-24, glp Python/fit-np-ul.py:45-48); what changes
-// is how the work is handed out and how one evaluation hands over to the next:
+// Each row batch goes through BatchTile of eval_kernel.cuh (see there for the lane mapping and
+// the reference lines: ll Python/fit-numpy.py:23-24, glp Python/fit-np-ul.py:45-48), as in the
+// static kernel; what changes is how the work is handed out and how one evaluation hands over
+// to the next:
 //
 //   * Dynamic row-batch scheduling.  Per-SM streaming rates differ (measured: the slowest 48
 //     CTAs of a 296-CTA grid finish 15-22 % after the median on one box, 4 % on another), so
@@ -73,22 +74,8 @@ __device__ __forceinline__ bool wait_epoch(const unsigned long long* epoch, unsi
 
 template <typename T, int P, bool GRAD>
 __global__ void __launch_bounds__(kBlock, 2) eval_persist_kernel(const EvalArgs a, const PersistArgs pa) {
-  using C = Chunk<T>;
-  using vec = typename C::vec;
-  using A = typename C::acc_t;
-  constexpr int V = C::V;
-  constexpr int CPR = P / V;
-  constexpr int L = CPR < 32 ? CPR : 32;
-  constexpr int SPR = CPR / L;
-  constexpr int G = 32 / L;
-  constexpr int S = 16;
-  constexpr int SG = S / SPR;
-  constexpr int RB = SG * G;
-  constexpr int LOG_L = ilog2(L), LOG_SG = ilog2(SG);
-  constexpr int NH = LOG_L < LOG_SG ? LOG_L : LOG_SG;
-  constexpr int M = SG >> NH;
-  static_assert(S % SPR == 0 && SG >= 1, "row too wide for the batch");
-  static_assert((1 << LOG_L) == L && (1 << LOG_SG) == SG, "power-of-two tiling");
+  using Tile = BatchTile<T, P>;
+  using vec = typename Tile::vec;
 
   __shared__ double red[kWarps][P + 1];   // [.][0] = log-likelihood, [.][1+c] = gradient column c
   __shared__ double tot[P + 1];
@@ -110,47 +97,26 @@ __global__ void __launch_bounds__(kBlock, 2) eval_persist_kernel(const EvalArgs 
   if (tid < kPoolSlots) s_tag[tid] = 0u;
   for (int j = tid; j < a.fin.p; j += kBlock) { s_ps[j] = a.fin.pscale[j]; s_lps[j] = a.fin.log_pscale[j]; }
   __syncthreads();
-  const int t_in_row = lane & (L - 1);
-  const int g_in_slab = lane >> LOG_L;
+  const Tile tl(a.n, lane);
   const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
-  const long long n = a.n;
-  const long long total_chunks = n * CPR;
-  const long long nbatch = (n + RB - 1) / RB;
+  const long long nbatch = tl.nbatch;
   const long long nwarps = (long long)gridDim.x * kWarps;
   const long long bt0 = (long long)blockIdx.x * kWarps + warp;
   // static prefix: KS batches per warp (strided), the rest is claimed dynamically from dyn0 on
   const long long KS = (nbatch / nwarps) * pa.static_eighths / 8;
   const long long dyn0 = KS * nwarps;
 
-  int khigh = 0;
-#pragma unroll
-  for (int b = 0; b < NH; ++b) khigh += ((t_in_row >> b) & 1) * (SG >> (b + 1));
-  const bool owner = (t_in_row >> NH) == 0;
-
   // stable at launch: nobody can complete evaluation 0 before every warp has passed this read
   const unsigned long long e0 = ld_acquire_gpu(pa.epoch);
 
-  vec v[S];
-  auto load_batch = [&](long long bt) {
-    const long long chunk0 = bt * (S * 32) + lane;
-    if (bt * RB + RB <= n) {
-#pragma unroll
-      for (int s = 0; s < S; ++s) v[s] = ldg_stream(Xv + chunk0 + s * 32);
-    } else {
-#pragma unroll
-      for (int s = 0; s < S; ++s) {
-        const long long c = chunk0 + s * 32;
-        v[s] = c < total_chunks ? ldg_stream(Xv + c) : zero_vec((vec*)nullptr);
-      }
-    }
-  };
+  vec v[Tile::S];
 
   for (int e = 0; e < pa.n_evals; ++e) {
     unsigned int* work = pa.work + ((e0 + (unsigned long long)e) & 1ull);
     EV_STAMP(0);
     long long cur = bt0;
     bool loaded = false;
-    if (KS > 0) { load_batch(cur); loaded = true; }   // X is immutable: fetch before beta is known
+    if (KS > 0) { tl.load(v, Xv, cur); loaded = true; }   // X is immutable: fetch before beta is known
 
     if (e > 0 && !wait_epoch(pa.epoch, e0 + (unsigned long long)e, pa.abort, pa.spin_limit_ns)) return;
     EV_STAMP(1);
@@ -199,93 +165,24 @@ __global__ void __launch_bounds__(kBlock, 2) eval_persist_kernel(const EvalArgs 
       sampler_precompute_draws(&s_st, a.fin.state);
     }
 
-    A bh[SPR][V];
-    float bl[SPR][V];
-#pragma unroll
-    for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int col = (sl * L + t_in_row) * V + i;
-        const double b = col < a.fin.p ? __ldcg(a.fin.beta + col) : 0.0;
-        bh[sl][i] = (A)b;
-        bl[sl][i] = (float)(b - (double)bh[sl][i]);
-      }
-
-    double acc[SPR][V];
-#pragma unroll
-    for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-      for (int i = 0; i < V; ++i) acc[sl][i] = 0.0;
+    typename Tile::Coef cf;
+    tl.load_coef(cf, a.fin.beta, a.fin.p);
+    double acc[Tile::SPR][Tile::V] = {};
     double ll_acc = 0.0;
 
     long long ks = 0;
     if (KS == 0) cur = next_dynamic();
     while (cur < nbatch) {
-      const long long row0 = cur * RB;
-      if (!loaded) load_batch(cur);
+      if (!loaded) tl.load(v, Xv, cur);
       loaded = false;
       // the index of the batch after this one, while the loads are in flight: static stride as
       // long as the prefix lasts, then a draw from the pool
       ++ks;
       if (tid == 0) producer_visit();
       const long long nxt = ks < KS ? bt0 + ks * nwarps : next_dynamic();
-      bool y1[M], valid[M];
-#pragma unroll
-      for (int j = 0; j < M; ++j) {
-        const long long row = row0 + (long long)(j + khigh) * G + g_in_slab;
-        valid[j] = owner && row < n;
-        y1[j] = valid[j] ? (a.y[row] != 0) : false;
-      }
-      A q[SG];
-#pragma unroll
-      for (int k = 0; k < SG; ++k) {
-        A s_hi = (A)0;
-#pragma unroll
-        for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-          for (int i = 0; i < V; ++i) s_hi = fma(elem(v[k * SPR + sl], i), bh[sl][i], s_hi);
-        if constexpr (sizeof(T) == 4) {
-          float s_lo = 0.f;
-#pragma unroll
-          for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-            for (int i = 0; i < V; ++i) s_lo = fmaf((float)elem(v[k * SPR + sl], i), bl[sl][i], s_lo);
-          s_hi += (A)s_lo;
-        }
-        q[k] = s_hi;
-      }
-      reduce_rows<SG, 0, LOG_L>(q, lane);
-      A r[M];
-#pragma unroll
-      for (int j = 0; j < M; ++j) {
-        A rr;
-        const A lt = row_terms(q[j], y1[j], rr);
-        r[j] = rr;
-        if (valid[j]) ll_acc += (double)lt;
-      }
-      if constexpr (GRAD) {
-        A gb[SPR][V];
-#pragma unroll
-        for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-          for (int i = 0; i < V; ++i) gb[sl][i] = (A)0;
-#pragma unroll
-        for (int k = 0; k < SG; ++k) {
-          const int j = k & (M - 1);
-          int tsrc = 0;
-#pragma unroll
-          for (int b = 0; b < NH; ++b) tsrc |= ((k >> (LOG_SG - 1 - b)) & 1) << b;
-          const A rr = __shfl_sync(0xffffffffu, r[j], (lane & ~(L - 1)) | tsrc);
-#pragma unroll
-          for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-            for (int i = 0; i < V; ++i) gb[sl][i] = fma(rr, (A)elem(v[k * SPR + sl], i), gb[sl][i]);
-        }
-#pragma unroll
-        for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-          for (int i = 0; i < V; ++i) acc[sl][i] += (double)gb[sl][i];
-      }
+      typename Tile::Rows rw;
+      tl.load_rows(rw, a.y, cur);
+      tl.template accumulate<GRAD>(v, rw, cf, ll_acc, acc);
       cur = nxt;
     }
     // The producer may leave the loop only once the END of the pool is published.  It normally gets
@@ -300,17 +197,7 @@ __global__ void __launch_bounds__(kBlock, 2) eval_persist_kernel(const EvalArgs 
     EV_STAMP(2);
 
     // ---- CTA reduction -> running sums
-    if constexpr (GRAD) {
-#pragma unroll
-      for (int sl = 0; sl < SPR; ++sl)
-#pragma unroll
-        for (int i = 0; i < V; ++i) {
-          double x = acc[sl][i];
-#pragma unroll
-          for (int o = L; o < 32; o <<= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-          if (lane < L) red[warp][1 + (sl * L + lane) * V + i] = x;
-        }
-    }
+    if constexpr (GRAD) tl.store_grad(acc, red[warp] + 1);
     ll_acc = warp_sum(ll_acc);
     if (lane == 0) red[warp][0] = ll_acc;
     __syncthreads();

@@ -78,20 +78,14 @@ struct LoglikArgs {
 
 template <typename T, int P>
 __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) loglik_kernel(const LoglikArgs a) {
-  using vec = typename Chunk<T>::vec;
-  constexpr int V = Chunk<T>::V;
-  constexpr int CPR = P / V;
-  constexpr int KC = P < 64 ? P : 64;
-  constexpr int DV = kPredDraws / V;
   extern __shared__ __align__(16) unsigned char ll_smem[];
   T* Xs = reinterpret_cast<T*>(ll_smem);     // [P][kPredLd]: X tile, (coefficient, row)
-  T* Bs = Xs + P * kPredLd;                  // [KC][kPredLd]: draw chunk, (coefficient, draw)
+  T* Bs = Xs + P * kPredLd;                  // [min(P, 64)][kPredLd]: draw chunk, (coefficient, draw)
 
   const int tid = threadIdx.x, tr = tid >> 4, td = tid & 15;
   const long long n = a.n, S = a.S;
   const long long ntiles = (n + kPredRows - 1) / kPredRows;
   const int ndt = (int)(a.Spad / kPredDraws);
-  const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
   const T* __restrict__ Bg = reinterpret_cast<const T*>(a.B);
 
   // work item = (row tile, group of kLoglikGroup draw tiles): the outputs are independent, so a
@@ -101,46 +95,11 @@ __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) loglik_kernel(
     const long long tile = w / ngroups;
     const int dt0 = (int)(w % ngroups) * kLoglikGroup, dt1 = min(dt0 + kLoglikGroup, ndt);
     const long long row0 = tile * kPredRows;
-    __syncthreads();
-    for (int idx = tid; idx < kPredRows * CPR; idx += kBlock) {
-      const int r = idx / CPR, c = idx % CPR;
-      const long long row = row0 + r;
-      const vec v = row < n ? ldg_stream(Xv + row * CPR + c) : zero_vec((vec*)nullptr);
-#pragma unroll
-      for (int i = 0; i < V; ++i) Xs[(c * V + i) * kPredLd + r] = elem(v, i);
-    }
-    unsigned ybits = 0;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const long long row = row0 + tr * 4 + i;
-      if (row < n && a.y[row] != 0) ybits |= 1u << i;
-    }
+    const unsigned ybits = stage_x_tile<T, P>(Xs, a.X, a.y, n, row0, tid, tr);
 
     for (int dt = dt0; dt < dt1; ++dt) {
       T eta[4][4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) eta[i][j] = (T)0;
-      for (int k0 = 0; k0 < P; k0 += KC) {
-        __syncthreads();
-        for (int idx = tid; idx < KC * DV; idx += kBlock) {
-          const int k = idx / DV, dv = idx % DV;
-          *reinterpret_cast<vec*>(Bs + k * kPredLd + dv * V) =
-              *reinterpret_cast<const vec*>(Bg + (long long)(k0 + k) * a.Spad + (long long)dt * kPredDraws + dv * V);
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (int k = 0; k < KC; ++k) {
-          T xv[4], bv[4];
-          lds4(Xs + (k0 + k) * kPredLd + tr * 4, xv);
-          lds4(Bs + k * kPredLd + td * 4, bv);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) eta[i][j] = fma(xv[i], bv[j], eta[i][j]);
-        }
-      }
+      draw_tile_eta<T, P>(eta, Xs, Bs, Bg, a.Spad, dt, tid, tr, td);
       const long long d0 = (long long)dt * kPredDraws + td * 4;
 #pragma unroll
       for (int i = 0; i < 4; ++i) {

@@ -12,6 +12,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/logreg_b200.h"
@@ -91,15 +92,17 @@ KernelChoice choice() {
   return k;
 }
 
-template <typename T>
-bool pick_p(int P, KernelChoice& k) {
+// f(std::integral_constant<int, P>()) for a padded width P the kernels are instantiated for;
+// false for any other width.
+template <typename F>
+bool with_width(int P, F&& f) {
   switch (P) {
-    case 8: k = choice<T, 8>(); return true;
-    case 16: k = choice<T, 16>(); return true;
-    case 32: k = choice<T, 32>(); return true;
-    case 64: k = choice<T, 64>(); return true;
-    case 128: k = choice<T, 128>(); return true;
-    case 256: k = choice<T, 256>(); return true;
+    case 8: f(std::integral_constant<int, 8>()); return true;
+    case 16: f(std::integral_constant<int, 16>()); return true;
+    case 32: f(std::integral_constant<int, 32>()); return true;
+    case 64: f(std::integral_constant<int, 64>()); return true;
+    case 128: f(std::integral_constant<int, 128>()); return true;
+    case 256: f(std::integral_constant<int, 256>()); return true;
   }
   return false;
 }
@@ -318,7 +321,10 @@ void apply_l2_policy(lrb_handle* h) {
 
 // choose kernels and grid for the bound shape
 int configure(lrb_handle* h) {
-  bool ok = h->mode == LRB_MODE_FP32 ? pick_p<float>(h->P, h->kern) : pick_p<double>(h->P, h->kern);
+  const bool fp32 = h->mode == LRB_MODE_FP32;
+  const bool ok = with_width(h->P, [&](auto w) {
+    h->kern = fp32 ? choice<float, decltype(w)::value>() : choice<double, decltype(w)::value>();
+  });
   if (!ok) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", h->P);
   int occ = 0, occ2 = 0;
   CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, h->kern.grad, kBlock, 0));
@@ -433,17 +439,33 @@ bool drive_ok(const lrb_handle* h, bool want_grad) {
   return (want_grad ? h->grid_drive : h->grid_drive_nograd) > 0;
 }
 
-// Drive mode: ONE cooperative launch performs `n_evals` consecutive evaluations (dynamic batch
-// scheduling; with a sampler state the last CTA of each evaluation produces the next point).
-int enqueue_drive(lrb_handle* h, const double* beta, SamplerState* st, bool want_grad, int n_evals) {
+// The arguments of the static and the drive-mode kernel for one evaluation at `beta` (device).
+// Row-sharded with NCCL the kernel only writes its sums, and finish_unfused completes the evaluation.
+EvalArgs eval_args(lrb_handle* h, const double* beta, SamplerState* st) {
   EvalArgs a{};
   a.X = h->X; a.y = h->y; a.n = h->n;
   a.partials = h->partials; a.ticket = h->ticket; a.sums = h->sums;
   a.fin = finish_args(h, beta, st);
   a.timeline = h->timeline;
-  const bool nccl_mode = (h->comm == 1 && h->world > 1);
-  a.fuse_finish = nccl_mode ? 0 : 1;
-  if (nccl_mode && n_evals != 1) return fail(h, LRB_E_STATE, "drive mode with NCCL takes one evaluation per launch (internal error)");
+  a.fuse_finish = (h->comm == 1 && h->world > 1) ? 0 : 1;
+  return a;
+}
+
+// After a kernel that did not run the finish step: NCCL allreduce of the sums, then finish_kernel.
+int finish_unfused(lrb_handle* h, const EvalArgs& a) {
+  if (a.fuse_finish) return LRB_OK;
+  CKN(h, g_nccl.AllReduce(h->sums, h->sums, (size_t)h->p + 1, ncclDouble, ncclSum, h->nccl, h->stream));
+  finish_kernel<<<1, kBlock, 0, h->stream>>>(a.fin, h->sums);
+  CK(h, cudaGetLastError());
+  h->kernel_launches++;
+  return LRB_OK;
+}
+
+// Drive mode: ONE cooperative launch performs `n_evals` consecutive evaluations (dynamic batch
+// scheduling; with a sampler state the last CTA of each evaluation produces the next point).
+int enqueue_drive(lrb_handle* h, const double* beta, SamplerState* st, bool want_grad, int n_evals) {
+  EvalArgs a = eval_args(h, beta, st);
+  if (!a.fuse_finish && n_evals != 1) return fail(h, LRB_E_STATE, "drive mode with NCCL takes one evaluation per launch (internal error)");
   PersistArgs pa{};
   pa.epoch = h->epoch; pa.work = h->work; pa.acc = h->drive_acc; pa.abort = h->drive_abort;
   pa.n_evals = n_evals; pa.spin_limit_ns = h->drive_spin_ns;
@@ -462,13 +484,7 @@ int enqueue_drive(lrb_handle* h, const double* beta, SamplerState* st, bool want
   }
   h->kernel_launches++;
   h->eval_launches += n_evals;
-  if (nccl_mode) {
-    CKN(h, g_nccl.AllReduce(h->sums, h->sums, (size_t)h->p + 1, ncclDouble, ncclSum, h->nccl, h->stream));
-    finish_kernel<<<1, kBlock, 0, h->stream>>>(a.fin, h->sums);
-    CK(h, cudaGetLastError());
-    h->kernel_launches++;
-  }
-  return LRB_OK;
+  return finish_unfused(h, a);
 }
 
 // After a synchronisation: did a drive-mode launch abandon a wait?  Leaves the counters clean.
@@ -492,17 +508,7 @@ int enqueue_eval(lrb_handle* h, const double* beta, SamplerState* st, bool want_
     if (rc == LRB_OK || !h->drive_launch_failed) return rc;
     // the cooperative launch was refused before anything ran: use the static kernel instead
   }
-  EvalArgs a{};
-  a.X = h->X;
-  a.y = h->y;
-  a.n = h->n;
-  a.partials = h->partials;
-  a.ticket = h->ticket;
-  a.sums = h->sums;
-  a.fin = finish_args(h, beta, st);
-  a.timeline = h->timeline;
-  const bool nccl_mode = (h->comm == 1 && h->world > 1);
-  a.fuse_finish = nccl_mode ? 0 : 1;
+  const EvalArgs a = eval_args(h, beta, st);
   EvalFn fn = want_grad ? h->kern.grad : h->kern.nograd;
   const int grid = want_grad ? h->grid : h->grid_nograd;
   if (h->pdl && h->world == 1) {   // measured: helps single-GPU small-n loops, neutral-to-negative with the peer exchange
@@ -521,13 +527,7 @@ int enqueue_eval(lrb_handle* h, const double* beta, SamplerState* st, bool want_
   CK(h, cudaGetLastError());
   h->kernel_launches++;
   h->eval_launches++;
-  if (nccl_mode) {
-    CKN(h, g_nccl.AllReduce(h->sums, h->sums, (size_t)h->p + 1, ncclDouble, ncclSum, h->nccl, h->stream));
-    finish_kernel<<<1, kBlock, 0, h->stream>>>(a.fin, h->sums);
-    CK(h, cudaGetLastError());
-    h->kernel_launches++;
-  }
-  return LRB_OK;
+  return finish_unfused(h, a);
 }
 
 template <typename ST, typename T>
@@ -1101,25 +1101,9 @@ extern "C" int lrb_lprior(lrb_handle* h, const double* beta, int C, double* out)
 namespace {
 
 using PredFn = void (*)(const PredictiveArgs);
-
-template <typename T, int P>
-PredFn predictive_for(size_t& smem) {
-  smem = predictive_smem<T, P>();
-  return predictive_kernel<T, P>;
-}
-
-template <typename T>
-PredFn pick_predictive(int P, size_t& smem) {
-  switch (P) {
-    case 8: return predictive_for<T, 8>(smem);
-    case 16: return predictive_for<T, 16>(smem);
-    case 32: return predictive_for<T, 32>(smem);
-    case 64: return predictive_for<T, 64>(smem);
-    case 128: return predictive_for<T, 128>(smem);
-    case 256: return predictive_for<T, 256>(smem);
-  }
-  return nullptr;
-}
+using LoglikFn = void (*)(const LoglikArgs);
+const auto predictive_pick = [](auto t, auto w) -> PredFn { return predictive_kernel<decltype(t), decltype(w)::value>; };
+const auto loglik_pick = [](auto t, auto w) -> LoglikFn { return loglik_kernel<decltype(t), decltype(w)::value>; };
 
 // draws (S x p, float64, row-major, host) -> dst: P x Spad in the mode's dtype, k-major, zero padded
 template <typename T>
@@ -1132,6 +1116,42 @@ int upload_draws(lrb_handle* h, void* dst, const double* draws, long long S, lon
   return LRB_OK;
 }
 
+// The draws of one call, uploaded for predictive_kernel or loglik_kernel (both read the same
+// layout and dynamic shared memory), and the launch shape of the kernel Fn.
+template <typename Fn>
+struct Draws {
+  DevTmp dB;
+  Fn fn = nullptr;
+  size_t smem = 0;
+  int occ = 0;
+  long long S = 0, Spad = 0;
+};
+
+// pick(T(), std::integral_constant<int, P>()) is the kernel for dtype T and padded width P.
+template <typename Fn, typename Pick>
+int draws_prepare(lrb_handle* h, const char* what, Pick pick, const double* draws, long long S, Draws<Fn>& g) {
+  const bool fp32 = h->mode == LRB_MODE_FP32;
+  const bool ok = with_width(h->P, [&](auto w) {
+    g.fn = fp32 ? pick(float(), w) : pick(double(), w);
+    g.smem = fp32 ? predictive_smem<float, decltype(w)::value>() : predictive_smem<double, decltype(w)::value>();
+  });
+  if (!ok) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", h->P);
+  CK(h, cudaFuncSetAttribute((const void*)g.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
+  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g.occ, g.fn, kBlock, g.smem));
+  if (g.occ < 1) return fail(h, LRB_E_CUDA, "%s kernel does not fit an SM", what);
+  g.S = S;
+  g.Spad = (S + kPredDraws - 1) / kPredDraws * kPredDraws;
+  CK(h, g.dB.alloc((size_t)h->P * g.Spad * (fp32 ? 4 : 8)));
+  return fp32 ? upload_draws<float>(h, g.dB.p, draws, S, g.Spad) : upload_draws<double>(h, g.dB.p, draws, S, g.Spad);
+}
+
+int check_single_gpu(lrb_handle* h, const char* what) {
+  if (h->world > 1)
+    return fail(h, LRB_E_UNSUPPORTED, "%s works on single-GPU handles only: this handle is rank %d of a row-sharded "
+                "group of %d, and its per-shard totals would need a collective", what, h->rank, h->world);
+  return LRB_OK;
+}
+
 }  // namespace
 
 extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int location, double* prob_mean,
@@ -1141,29 +1161,15 @@ extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int
   if (!draws || S < 1) return fail(h, LRB_E_BAD_ARG, "draws is NULL or S < 1 (S=%lld)", (long long)S);
   if (S > (1ll << 30)) return fail(h, LRB_E_BAD_ARG, "S=%lld draws exceeds 2^30", (long long)S);
   if (location != LRB_HOST && location != LRB_DEVICE) return fail(h, LRB_E_BAD_ARG, "bad location %d", location);
-  if (h->world > 1)
-    return fail(h, LRB_E_UNSUPPORTED, "lrb_predictive works on single-GPU handles only: this handle is rank %d of a "
-                "row-sharded group of %d, and its per-shard totals would need a collective", h->rank, h->world);
+  if (int rc = check_single_gpu(h, "lrb_predictive")) return rc;
   if (use_device(h)) return LRB_E_CUDA;
-  const bool fp32 = h->mode == LRB_MODE_FP32;
-  const int P = h->P;
-  size_t smem = 0;
-  PredFn fn = fp32 ? pick_predictive<float>(P, smem) : pick_predictive<double>(P, smem);
-  if (!fn) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", P);
-  CK(h, cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int occ = 0;
-  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kBlock, smem));
-  if (occ < 1) return fail(h, LRB_E_CUDA, "predictive kernel does not fit an SM");
+  Draws<PredFn> g;
+  if (int rc = draws_prepare(h, "predictive", predictive_pick, draws, S, g)) return rc;
   const long long ntiles = (h->n + kPredRows - 1) / kPredRows;
-  const int grid = (int)std::min<long long>((long long)h->sms * occ, ntiles);
-  const long long Spad = (S + kPredDraws - 1) / kPredDraws * kPredDraws;
+  const int grid = (int)std::min<long long>((long long)h->sms * g.occ, ntiles);
 
-  // scratch: draws, CTA partials, totals, ticket; per-row outputs on the device when the caller's are on the host
-  DevTmp dB, work, out[4];
-  const size_t es = fp32 ? 4 : 8;
-  CK(h, dB.alloc((size_t)P * Spad * es));
-  int rc = fp32 ? upload_draws<float>(h, dB.p, draws, S, Spad) : upload_draws<double>(h, dB.p, draws, S, Spad);
-  if (rc) return rc;
+  // scratch: CTA partials, totals, ticket; per-row outputs on the device when the caller's are on the host
+  DevTmp work, out[4];
   const size_t wdoubles = (size_t)grid * kPredPartial + kPredTotals;
   CK(h, work.alloc(wdoubles * sizeof(double) + sizeof(unsigned int)));
   unsigned int* ticket = reinterpret_cast<unsigned int*>(work.as<double>() + wdoubles);
@@ -1179,12 +1185,12 @@ extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int
 
   PredictiveArgs a{};
   a.X = h->X; a.y = h->y; a.n = h->n;
-  a.B = dB.p; a.S = S; a.Spad = Spad;
+  a.B = g.dB.p; a.S = S; a.Spad = g.Spad;
   a.prob_mean = dev[0]; a.prob_sd = dev[1]; a.lppd = dev[2]; a.p_waic = dev[3];
   a.partials = work.as<double>();
   a.ticket = ticket;
   a.totals = work.as<double>() + (size_t)grid * kPredPartial;
-  fn<<<grid, kBlock, smem, h->stream>>>(a);
+  g.fn<<<grid, kBlock, g.smem, h->stream>>>(a);
   CK(h, cudaGetLastError());
   h->kernel_launches++;
 
@@ -1208,45 +1214,8 @@ extern "C" int lrb_predictive(lrb_handle* h, const double* draws, int64_t S, int
 // ============================================================ PSIS-LOO / pointwise log-likelihood
 namespace {
 
-using LoglikFn = void (*)(const LoglikArgs);
-
-template <typename T>
-LoglikFn pick_loglik(int P, size_t& smem) {
-  switch (P) {
-    case 8: smem = predictive_smem<T, 8>(); return loglik_kernel<T, 8>;
-    case 16: smem = predictive_smem<T, 16>(); return loglik_kernel<T, 16>;
-    case 32: smem = predictive_smem<T, 32>(); return loglik_kernel<T, 32>;
-    case 64: smem = predictive_smem<T, 64>(); return loglik_kernel<T, 64>;
-    case 128: smem = predictive_smem<T, 128>(); return loglik_kernel<T, 128>;
-    case 256: smem = predictive_smem<T, 256>(); return loglik_kernel<T, 256>;
-  }
-  return nullptr;
-}
-
-// Stage 1 for one handle and one set of draws: the uploaded draws and the kernel's launch shape.
-struct Loglik {
-  DevTmp dB;
-  LoglikFn fn = nullptr;
-  size_t smem = 0;
-  int occ = 0;
-  long long S = 0, Spad = 0;
-};
-
-int loglik_prepare(lrb_handle* h, const double* draws, long long S, Loglik& g) {
-  const bool fp32 = h->mode == LRB_MODE_FP32;
-  g.fn = fp32 ? pick_loglik<float>(h->P, g.smem) : pick_loglik<double>(h->P, g.smem);
-  if (!g.fn) return fail(h, LRB_E_UNSUPPORTED, "unsupported padded column count %d", h->P);
-  CK(h, cudaFuncSetAttribute((const void*)g.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
-  CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&g.occ, g.fn, kBlock, g.smem));
-  if (g.occ < 1) return fail(h, LRB_E_CUDA, "log-likelihood kernel does not fit an SM");
-  g.S = S;
-  g.Spad = (S + kPredDraws - 1) / kPredDraws * kPredDraws;
-  CK(h, g.dB.alloc((size_t)h->P * g.Spad * (fp32 ? 4 : 8)));
-  return fp32 ? upload_draws<float>(h, g.dB.p, draws, S, g.Spad) : upload_draws<double>(h, g.dB.p, draws, S, g.Spad);
-}
-
 // L[i][s] (row stride S) for the bound rows [row0, row0 + rows)
-int loglik_launch(lrb_handle* h, const Loglik& g, long long row0, long long rows, double* L) {
+int loglik_launch(lrb_handle* h, const Draws<LoglikFn>& g, long long row0, long long rows, double* L) {
   const size_t es = h->mode == LRB_MODE_FP32 ? 4 : 8;
   LoglikArgs a{};
   a.X = static_cast<const char*>(h->X) + (size_t)row0 * h->P * es;
@@ -1273,13 +1242,6 @@ long long loo_chunk_rows(long long n, long long S) {
   return std::min<long long>(R, (n + kPredRows - 1) / kPredRows * kPredRows);
 }
 
-int check_single_gpu(lrb_handle* h, const char* what) {
-  if (h->world > 1)
-    return fail(h, LRB_E_UNSUPPORTED, "%s works on single-GPU handles only: this handle is rank %d of a row-sharded "
-                "group of %d, and its per-shard totals would need a collective", what, h->rank, h->world);
-  return LRB_OK;
-}
-
 }  // namespace
 
 extern "C" int lrb_loglik(lrb_handle* h, const double* draws, int64_t S, int64_t row0, int64_t nrows, int location,
@@ -1294,8 +1256,8 @@ extern "C" int lrb_loglik(lrb_handle* h, const double* draws, int64_t S, int64_t
   if (location != LRB_HOST && location != LRB_DEVICE) return fail(h, LRB_E_BAD_ARG, "bad location %d", location);
   if (int rc = check_single_gpu(h, "lrb_loglik")) return rc;
   if (use_device(h)) return LRB_E_CUDA;
-  Loglik g;
-  if (int rc = loglik_prepare(h, draws, S, g)) return rc;
+  Draws<LoglikFn> g;
+  if (int rc = draws_prepare(h, "log-likelihood", loglik_pick, draws, S, g)) return rc;
   if (location == LRB_DEVICE) {
     if (int rc = loglik_launch(h, g, row0, nrows, out)) return rc;
   } else {   // chunk by chunk through a bounded device buffer
@@ -1325,8 +1287,8 @@ extern "C" int lrb_loo(lrb_handle* h, const double* draws, int64_t S, int locati
   if (int rc = check_single_gpu(h, "lrb_loo")) return rc;
   if (use_device(h)) return LRB_E_CUDA;
   const bool stage2 = !getenv("LRB_LOO_STAGE1_ONLY");   // timing of stage 1 alone (header, tools/loo_bench.py)
-  Loglik g;
-  if (int rc = loglik_prepare(h, draws, S, g)) return rc;
+  Draws<LoglikFn> g;
+  if (int rc = draws_prepare(h, "log-likelihood", loglik_pick, draws, S, g)) return rc;
   const long long n = h->n, M = psis_tail_len(S);
   const int stage = S <= kLooRowSmem ? 1 : 0;
   const size_t smem = psis_smem(S, M, stage);

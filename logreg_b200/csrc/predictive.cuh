@@ -84,6 +84,66 @@ __device__ __forceinline__ void lds4(const double* p, double (&v)[4]) {
   v[0] = a.x; v[1] = a.y; v[2] = b.x; v[3] = b.y;
 }
 
+// Rows row0..+63 into Xs, transposed ([coefficient][row], zero past n), after a barrier that
+// frees Xs of the previous tile.  Returns the labels of row group tr's 4 rows as bits.
+template <typename T, int P>
+__device__ __forceinline__ unsigned stage_x_tile(T* Xs, const void* X, const uint8_t* y, long long n, long long row0,
+                                                 int tid, int tr) {
+  using vec = typename Chunk<T>::vec;
+  constexpr int V = Chunk<T>::V;
+  constexpr int CPR = P / V;                 // 16-byte chunks per row of X
+  const vec* __restrict__ Xv = reinterpret_cast<const vec*>(X);
+  __syncthreads();   // every thread is done with the previous tile's X
+  for (int idx = tid; idx < kPredRows * CPR; idx += kBlock) {
+    const int r = idx / CPR, c = idx % CPR;
+    const long long row = row0 + r;
+    const vec v = row < n ? ldg_stream(Xv + row * CPR + c) : zero_vec((vec*)nullptr);
+#pragma unroll
+    for (int i = 0; i < V; ++i) Xs[(c * V + i) * kPredLd + r] = elem(v, i);
+  }
+  unsigned ybits = 0;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const long long row = row0 + tr * 4 + i;
+    if (row < n && y[row] != 0) ybits |= 1u << i;
+  }
+  return ybits;
+}
+
+// eta[i][j] = x(row tr*4 + i of the tile in Xs) . beta(draw dt*64 + td*4 + j), the draws (P x Spad,
+// k-major in Bg) staged through Bs in chunks of KC coefficients.
+template <typename T, int P>
+__device__ __forceinline__ void draw_tile_eta(T (&eta)[4][4], const T* Xs, T* Bs, const T* Bg, long long Spad, int dt,
+                                              int tid, int tr, int td) {
+  using vec = typename Chunk<T>::vec;
+  constexpr int V = Chunk<T>::V;
+  constexpr int KC = P < 64 ? P : 64;        // coefficients per chunk of draws in shared memory
+  constexpr int DV = kPredDraws / V;         // 16-byte chunks per 64 draws
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) eta[i][j] = (T)0;
+  for (int k0 = 0; k0 < P; k0 += KC) {
+    __syncthreads();   // the previous chunk is consumed (and, the first time, Xs is complete)
+    for (int idx = tid; idx < KC * DV; idx += kBlock) {
+      const int k = idx / DV, dv = idx % DV;
+      *reinterpret_cast<vec*>(Bs + k * kPredLd + dv * V) =
+          *reinterpret_cast<const vec*>(Bg + (long long)(k0 + k) * Spad + (long long)dt * kPredDraws + dv * V);
+    }
+    __syncthreads();
+#pragma unroll 4
+    for (int k = 0; k < KC; ++k) {
+      T xv[4], bv[4];
+      lds4(Xs + (k0 + k) * kPredLd + tr * 4, xv);
+      lds4(Bs + k * kPredLd + td * 4, bv);
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) eta[i][j] = fma(xv[i], bv[j], eta[i][j]);
+    }
+  }
+}
+
 // (n, mean, M2) of a into which b is merged (Chan, Golub & LeVeque).
 __device__ __forceinline__ void merge_moments(double& n, double& mean, double& m2, double nb, double meanb,
                                               double m2b) {
@@ -106,14 +166,9 @@ __device__ __forceinline__ void merge_lse(double& c, double& s, double m, double
 
 template <typename T, int P>
 __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) predictive_kernel(const PredictiveArgs a) {
-  using vec = typename Chunk<T>::vec;
-  constexpr int V = Chunk<T>::V;
-  constexpr int CPR = P / V;                 // 16-byte chunks per row of X
-  constexpr int KC = P < 64 ? P : 64;        // coefficients per chunk of draws in shared memory
-  constexpr int DV = kPredDraws / V;         // 16-byte chunks per 64 draws
   extern __shared__ __align__(16) unsigned char pred_smem[];
   T* Xs = reinterpret_cast<T*>(pred_smem);   // [P][kPredLd]: X tile, (coefficient, row)
-  T* Bs = Xs + P * kPredLd;                  // [KC][kPredLd]: draw chunk, (coefficient, draw)
+  T* Bs = Xs + P * kPredLd;                  // [min(P, 64)][kPredLd]: draw chunk, (coefficient, draw)
   __shared__ double s_own[16][kPredPartial];
   __shared__ T s_ref[3][4][kBlock];          // per thread and row: shifts of sigma and l, log-sum-exp reference c
   __shared__ double s_lse[4][kBlock];        // per thread and row: sum expm1(l - c)
@@ -123,7 +178,6 @@ __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) predictive_ker
   const long long n = a.n, S = a.S;
   const long long ntiles = (n + kPredRows - 1) / kPredRows;
   const int ndt = (int)(a.Spad / kPredDraws);
-  const vec* __restrict__ Xv = reinterpret_cast<const vec*>(a.X);
   const T* __restrict__ Bg = reinterpret_cast<const T*>(a.B);
   const double Sd = (double)S;
 
@@ -135,20 +189,7 @@ __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) predictive_ker
 
   for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     const long long row0 = tile * kPredRows;
-    __syncthreads();   // every thread is done with the previous tile's X
-    for (int idx = tid; idx < kPredRows * CPR; idx += kBlock) {
-      const int r = idx / CPR, c = idx % CPR;
-      const long long row = row0 + r;
-      const vec v = row < n ? ldg_stream(Xv + row * CPR + c) : zero_vec((vec*)nullptr);
-#pragma unroll
-      for (int i = 0; i < V; ++i) Xs[(c * V + i) * kPredLd + r] = elem(v, i);
-    }
-    unsigned ybits = 0;                      // labels of this thread's 4 rows
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const long long row = row0 + tr * 4 + i;
-      if (row < n && a.y[row] != 0) ybits |= 1u << i;
-    }
+    const unsigned ybits = stage_x_tile<T, P>(Xs, a.X, a.y, n, row0, tid, tr);   // labels of this thread's 4 rows
 
     // s_ref and s_lse are touched once per tile: registers are kept for the tile
     double s1s[4], s2s[4], s1l[4], s2l[4];
@@ -162,29 +203,7 @@ __global__ void __launch_bounds__(kBlock, sizeof(T) == 4 ? 2 : 1) predictive_ker
 
     for (int dt = 0; dt < ndt; ++dt) {
       T eta[4][4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) eta[i][j] = (T)0;
-      for (int k0 = 0; k0 < P; k0 += KC) {
-        __syncthreads();   // the previous chunk is consumed (and, the first time, Xs is complete)
-        for (int idx = tid; idx < KC * DV; idx += kBlock) {
-          const int k = idx / DV, dv = idx % DV;
-          *reinterpret_cast<vec*>(Bs + k * kPredLd + dv * V) =
-              *reinterpret_cast<const vec*>(Bg + (long long)(k0 + k) * a.Spad + (long long)dt * kPredDraws + dv * V);
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (int k = 0; k < KC; ++k) {
-          T xv[4], bv[4];
-          lds4(Xs + (k0 + k) * kPredLd + tr * 4, xv);
-          lds4(Bs + k * kPredLd + td * 4, bv);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j) eta[i][j] = fma(xv[i], bv[j], eta[i][j]);
-        }
-      }
+      draw_tile_eta<T, P>(eta, Xs, Bs, Bg, a.Spad, dt, tid, tr, td);
 
       // link functions and statistics: valid draws of this thread in this tile (< 4 only in the last)
       const long long d0 = (long long)dt * kPredDraws + td * 4;
