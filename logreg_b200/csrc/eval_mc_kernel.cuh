@@ -5,7 +5,8 @@
 // over, where eta = X B' and G = R' X become tensor-core contractions.
 //
 // Each chain's batch goes through BatchTile (eval_kernel.cuh), as in the single-chain kernels;
-// the finish step runs in a separate launch with one CTA per chain.
+// the finish step runs in a separate launch with one CTA per chain.  Chain c uses row c of the
+// handle's per-chain sums, result and state arrays; the single-chain kernels use row 0.
 #pragma once
 #include "eval_kernel.cuh"
 
@@ -110,18 +111,28 @@ __global__ void __launch_bounds__(kBlock, 1) eval_mc_kernel(const EvalMcArgs a) 
   }
 }
 
-// One CTA per chain: prior + result + sampler update from the reduced sums.
+// Chain c's finish arguments in a finish launch of its own (one CTA per chain): its state,
+// coefficients and result row.  Its sums are complete by then (an NCCL allreduce runs between the
+// launches), so there is no peer exchange.  false: the chain is paused and its CTA has nothing to do.
+__device__ inline bool chain_finish_args(FinishArgs& f, int c, SamplerState* states, const double* beta_base,
+                                         long long beta_stride, double* res) {
+  f.state = states ? states + c : nullptr;
+  if (f.state && f.state->phase == PH_PAUSED) return false;
+  f.beta = beta_base + (long long)c * beta_stride;
+  f.res = res + (size_t)c * kResStride;
+  f.p2p = 0;
+  return true;
+}
+
+// One CTA per chain: prior + result + sampler update from the reduced sums.  Also the finish of
+// a single-chain evaluation whose kernel left it out (row-sharded with NCCL).
 __global__ void finish_mc_kernel(FinishArgs base, const double* sums, SamplerState* states,
                                  const double* beta_base, long long beta_stride, double* res) {
   __shared__ double s_sums[kMaxP + 1];
   __shared__ double scratch[kWarps];
   const int c = blockIdx.x;
   FinishArgs f = base;
-  f.state = states ? states + c : nullptr;
-  if (f.state && f.state->phase == PH_PAUSED) return;
-  f.beta = beta_base + (long long)c * beta_stride;
-  f.res = res + (size_t)c * kResStride;
-  f.p2p = 0;
+  if (!chain_finish_args(f, c, states, beta_base, beta_stride, res)) return;
   for (int i = threadIdx.x; i <= f.p; i += kBlock) s_sums[i] = sums[(size_t)c * kSumStride + i];
   __syncthreads();
   finish_eval(f, s_sums, scratch);

@@ -506,11 +506,7 @@ __global__ void finish_tc_kernel(FinishArgs base, const double* partials, int ro
   __shared__ double scratch[kWarps];
   const int c = blockIdx.x;
   FinishArgs f = base;
-  f.state = states ? states + c : nullptr;
-  if (f.state && f.state->phase == PH_PAUSED) return;
-  f.beta = beta_base + (long long)c * beta_stride;
-  f.res = res + (size_t)c * kResStride;
-  f.p2p = 0;
+  if (!chain_finish_args(f, c, states, beta_base, beta_stride, res)) return;
   const int cg = c / kTcChains, ci = c % kTcChains;
   for (int j = threadIdx.x; j <= f.p; j += kBlock) {
     double s = 0.0;

@@ -135,9 +135,6 @@ struct lrb_handle {
   int grid = 0, grid_nograd = 0;
   double* partials = nullptr;
   unsigned int* ticket = nullptr;
-  double* sums = nullptr;   // [kMaxP+1]
-  double* res = nullptr;    // [kMaxP+3]
-  double* beta = nullptr;   // [kMaxP]
   double* pinned = nullptr; // host staging [2*kMaxP+8]
   // drive mode (eval_persist_kernel.cuh): one block of device words [epoch u64][work u32 x2][abort i32][pad][acc f64 x (kMaxP+1)]
   void* drive_mem = nullptr;
@@ -155,8 +152,6 @@ struct lrb_handle {
   int drive_static_eighths = -1;  // -1: chosen per shape in configure(); LRB_DRIVE_STATIC overrides
 
   // sampler
-  SamplerState* state = nullptr;
-  double* d_init = nullptr;   // [kMaxP]
   double* d_scale = nullptr;  // [kMaxP]
   double* d_out = nullptr; size_t out_cap = 0;
   double* d_z = nullptr; size_t z_cap = 0;
@@ -192,12 +187,12 @@ struct lrb_handle {
   bool peer_open[kMaxRanks] = {};
   long long p2p_timeout_ns = 60ll * 1000 * 1000 * 1000;
 
-  // many-chain (C >= 2) state
-  SamplerState* states_mc = nullptr;
-  double* sums_mc = nullptr;   // [C][kSumStride]
-  double* res_mc = nullptr;    // [C][kResStride]
-  double* beta_mc = nullptr;   // [C][kMaxP] staging for host coefficient / init matrices
-  int mc_cap = 0;
+  // per-chain arrays of chain_cap rows; a single chain or evaluation uses row 0
+  SamplerState* states = nullptr;
+  double* sums = nullptr;   // [C][kSumStride]
+  double* res = nullptr;    // [C][kResStride]
+  double* beta = nullptr;   // [C][kMaxP] staging for host coefficient / init matrices
+  int chain_cap = 0;
   int run_C = 1, chain_C = 1, graph_C = 1;
   int grid_mc = 0;
   long long graph_kl_per_replay = 0, graph_el_per_replay = 0;
@@ -451,11 +446,12 @@ EvalArgs eval_args(lrb_handle* h, const double* beta, SamplerState* st) {
   return a;
 }
 
-// After a kernel that did not run the finish step: NCCL allreduce of the sums, then finish_kernel.
+// After a kernel that did not run the finish step: NCCL allreduce of the sums, then the finish of
+// chain 0 in a launch of its own.
 int finish_unfused(lrb_handle* h, const EvalArgs& a) {
   if (a.fuse_finish) return LRB_OK;
   CKN(h, g_nccl.AllReduce(h->sums, h->sums, (size_t)h->p + 1, ncclDouble, ncclSum, h->nccl, h->stream));
-  finish_kernel<<<1, kBlock, 0, h->stream>>>(a.fin, h->sums);
+  finish_mc_kernel<<<1, kBlock, 0, h->stream>>>(a.fin, h->sums, a.fin.state, a.fin.beta, 0, h->res);
   CK(h, cudaGetLastError());
   h->kernel_launches++;
   return LRB_OK;
@@ -564,6 +560,39 @@ int alloc_data(lrb_handle* h, long long n, int p, int mode) {
   return LRB_OK;
 }
 
+// states / results / sums / coefficients for C chains
+int ensure_chains(lrb_handle* h, int C) {
+  if (C <= h->chain_cap) return LRB_OK;
+  // The launch graph bakes these pointers into its kernel arguments: it dies with the reallocation.
+  // So does a paused many-chain run; a paused or armed single chain carries on from row 0.
+  CK(h, cudaStreamSynchronize(h->stream));
+  drop_graph(h);
+  if (h->chain_C > 1) { h->chain_live = false; h->run_armed = false; }
+  // The old rows are copied before the old array is freed.  SamplerState holds no pointer into its
+  // own array (z, u, out and mom_* point into d_z, d_u, d_out and d_mom_*): a byte copy moves a row.
+  auto regrow = [&](auto*& buf, size_t row_bytes, bool zero) {
+    void* fresh = nullptr;
+    cudaError_t e = cudaMalloc(&fresh, (size_t)C * row_bytes);
+    if (e == cudaSuccess && zero) e = cudaMemsetAsync(fresh, 0, (size_t)C * row_bytes, h->stream);
+    if (e == cudaSuccess && buf)
+      e = cudaMemcpyAsync(fresh, buf, (size_t)h->chain_cap * row_bytes, cudaMemcpyDeviceToDevice, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) { cudaFree(fresh); return e; }
+    cudaFree(buf);
+    buf = static_cast<std::remove_reference_t<decltype(buf)>>(fresh);
+    return cudaSuccess;
+  };
+  // states last, so that lrb_create places the single-chain state right before the drive-mode words
+  // it allocates next: config 2 (drive mode) measured 0.6-0.8 % slower on a B200 (1000 W) with the
+  // state allocated first.
+  CK(h, regrow(h->sums, kSumStride * sizeof(double), false));
+  CK(h, regrow(h->res, kResStride * sizeof(double), false));
+  CK(h, regrow(h->beta, kMaxP * sizeof(double), false));
+  CK(h, regrow(h->states, sizeof(SamplerState), true));
+  h->chain_cap = C;
+  return LRB_OK;
+}
+
 }  // namespace
 
 // ============================================================ lifetime
@@ -607,13 +636,8 @@ extern "C" int lrb_create(int device, lrb_handle** out) {
   CKC(cudaMalloc(&h->partials, (size_t)h->sms * 8 * kMcChains * (kMaxP + 1) * sizeof(double)));
   CKC(cudaMalloc(&h->ticket, sizeof(unsigned int)));
   CKC(cudaMemset(h->ticket, 0, sizeof(unsigned int)));
-  CKC(cudaMalloc(&h->sums, (kMaxP + 1) * sizeof(double)));
-  CKC(cudaMalloc(&h->res, (kMaxP + 3) * sizeof(double)));
-  CKC(cudaMalloc(&h->beta, kMaxP * sizeof(double)));
-  CKC(cudaMalloc(&h->d_init, kMaxP * sizeof(double)));
   CKC(cudaMalloc(&h->d_scale, kMaxP * sizeof(double)));
-  CKC(cudaMalloc(&h->state, sizeof(SamplerState)));
-  CKC(cudaMemset(h->state, 0, sizeof(SamplerState)));
+  if (ensure_chains(h, 1)) return bail(LRB_E_CUDA);
   CKC(cudaMalloc(&h->seq, sizeof(unsigned long long)));
   CKC(cudaMemset(h->seq, 0, sizeof(unsigned long long)));
   CKC(cudaMalloc(&h->comm_error, sizeof(int)));
@@ -652,10 +676,9 @@ extern "C" int lrb_destroy(lrb_handle* h) {
   for (int r = 0; r < kMaxRanks; ++r)
     if (h->peer_open[r]) cudaIpcCloseMemHandle(h->peer_base[r]);
   free_data(h);
-  void* bufs[] = {h->d_pscale, h->d_logps, h->partials, h->ticket, h->sums, h->res, h->beta, h->d_init,
-                  h->d_scale, h->state, h->seq, h->comm_error, h->d_out, h->d_z, h->d_u, h->mailbox,
-                  h->states_mc, h->sums_mc, h->res_mc, h->beta_mc, h->partials_tc, h->timeline, h->drive_mem,
-                  h->d_mom_mean, h->d_mom_m2};
+  void* bufs[] = {h->d_pscale, h->d_logps, h->partials, h->ticket, h->d_scale, h->seq, h->comm_error,
+                  h->d_out, h->d_z, h->d_u, h->mailbox, h->states, h->sums, h->res, h->beta, h->partials_tc,
+                  h->timeline, h->drive_mem, h->d_mom_mean, h->d_mom_m2};
   for (void* b : bufs) if (b) cudaFree(b);
   if (h->pinned) cudaFreeHost(h->pinned);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -849,28 +872,6 @@ extern "C" int lrb_copy_rows(lrb_handle* h, int64_t row0, int64_t nrows, double*
 // ============================================================ evaluation
 namespace {
 
-// states / results / sums for C chains
-int ensure_chains(lrb_handle* h, int C) {
-  if (C <= h->mc_cap) return LRB_OK;
-  // The launch graph bakes these pointers into its kernel arguments and a paused many-chain run
-  // lives in states_mc: both die with the reallocation.
-  CK(h, cudaStreamSynchronize(h->stream));
-  drop_graph(h);
-  if (h->chain_C > 1) { h->chain_live = false; h->run_armed = false; }
-  if (h->states_mc) cudaFree(h->states_mc);
-  if (h->sums_mc) cudaFree(h->sums_mc);
-  if (h->res_mc) cudaFree(h->res_mc);
-  if (h->beta_mc) cudaFree(h->beta_mc);
-  h->states_mc = nullptr; h->sums_mc = nullptr; h->res_mc = nullptr; h->beta_mc = nullptr; h->mc_cap = 0;
-  CK(h, cudaMalloc(&h->states_mc, (size_t)C * sizeof(SamplerState)));
-  CK(h, cudaMemset(h->states_mc, 0, (size_t)C * sizeof(SamplerState)));
-  CK(h, cudaMalloc(&h->sums_mc, (size_t)C * kSumStride * sizeof(double)));
-  CK(h, cudaMalloc(&h->res_mc, (size_t)C * kResStride * sizeof(double)));
-  CK(h, cudaMalloc(&h->beta_mc, (size_t)C * kMaxP * sizeof(double)));
-  h->mc_cap = C;
-  return LRB_OK;
-}
-
 bool use_tc(const lrb_handle* h, int C) {
   return h->tc_ok && h->world == 1 && C >= h->tc_min_chains && (C + kTcChains - 1) / kTcChains <= h->sms;
 }
@@ -911,7 +912,7 @@ int enqueue_eval_tc(lrb_handle* h, const double* beta_base, long long beta_strid
   h->kernel_launches++;
   h->eval_launches++;
   FinishArgs f = finish_args(h, nullptr, nullptr);
-  finish_tc_kernel<<<C, kBlock, 0, h->stream>>>(f, h->partials_tc, gx, groups, h->P, states, beta_base, beta_stride, h->res_mc);
+  finish_tc_kernel<<<C, kBlock, 0, h->stream>>>(f, h->partials_tc, gx, groups, h->P, states, beta_base, beta_stride, h->res);
   CK(h, cudaGetLastError());
   h->kernel_launches++;
   return LRB_OK;
@@ -929,16 +930,16 @@ int enqueue_eval_mc(lrb_handle* h, const double* beta_base, long long beta_strid
     a.partials = h->partials; a.ticket = h->ticket;
     a.beta_base = beta_base; a.beta_stride = beta_stride;
     a.chain0 = c0; a.nc_active = std::min(NC, C - c0); a.p = h->p;
-    a.sums = h->sums_mc; a.states = states;
+    a.sums = h->sums; a.states = states;
     h->kern.mc<<<h->grid_mc, kBlock, 0, h->stream>>>(a);
     CK(h, cudaGetLastError());
     h->kernel_launches++;
     h->eval_launches++;
   }
   if (h->comm == 1 && h->world > 1)
-    CKN(h, g_nccl.AllReduce(h->sums_mc, h->sums_mc, (size_t)C * kSumStride, ncclDouble, ncclSum, h->nccl, h->stream));
+    CKN(h, g_nccl.AllReduce(h->sums, h->sums, (size_t)C * kSumStride, ncclDouble, ncclSum, h->nccl, h->stream));
   FinishArgs f = finish_args(h, nullptr, nullptr);
-  finish_mc_kernel<<<C, kBlock, 0, h->stream>>>(f, h->sums_mc, states, beta_base, beta_stride, h->res_mc);
+  finish_mc_kernel<<<C, kBlock, 0, h->stream>>>(f, h->sums, states, beta_base, beta_stride, h->res);
   CK(h, cudaGetLastError());
   h->kernel_launches++;
   return LRB_OK;
@@ -972,10 +973,10 @@ extern "C" int lrb_eval(lrb_handle* h, const double* beta, int C, int want_grad,
     int rc = ensure_chains(h, C);
     if (rc) return rc;
     if ((rc = reserve_tc(h, C))) return rc;
-    CK(h, cudaMemcpyAsync(h->beta_mc, beta, (size_t)C * p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    if ((rc = enqueue_eval_mc(h, h->beta_mc, p, C, nullptr))) return rc;
+    CK(h, cudaMemcpyAsync(h->beta, beta, (size_t)C * p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    if ((rc = enqueue_eval_mc(h, h->beta, p, C, nullptr))) return rc;
     std::vector<double> back((size_t)C * kResStride);
-    CK(h, cudaMemcpyAsync(back.data(), h->res_mc, back.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaMemcpyAsync(back.data(), h->res, back.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
     for (int c = 0; c < C; ++c) {
       const double* r = back.data() + (size_t)c * kResStride;
@@ -1018,8 +1019,8 @@ extern "C" int lrb_debug_tc_eta(lrb_handle* h, const double* beta, int C, float*
   const size_t cnt = (size_t)groups * kTcChains * kTcRows;
   CK(h, cudaMalloc(&h->dbg_eta, cnt * sizeof(float)));
   CK(h, cudaMemsetAsync(h->dbg_eta, 0, cnt * sizeof(float), h->stream));
-  cudaError_t e = cudaMemcpyAsync(h->beta_mc, beta, (size_t)C * h->p * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-  if (e == cudaSuccess) rc = enqueue_eval_tc(h, h->beta_mc, h->p, C, nullptr);
+  cudaError_t e = cudaMemcpyAsync(h->beta, beta, (size_t)C * h->p * sizeof(double), cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess) rc = enqueue_eval_tc(h, h->beta, h->p, C, nullptr);
   if (e == cudaSuccess && rc == LRB_OK) e = cudaMemcpyAsync(eta_out, h->dbg_eta, cnt * sizeof(float), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess && rc == LRB_OK) e = cudaStreamSynchronize(h->stream);
   cudaFree(h->dbg_eta);
@@ -1029,7 +1030,7 @@ extern "C" int lrb_debug_tc_eta(lrb_handle* h, const double* beta, int C, float*
     std::vector<long long> tl(64 * 16, 0);
     cudaMalloc(&h->dbg_time, tl.size() * sizeof(long long));
     cudaMemset(h->dbg_time, 0, tl.size() * sizeof(long long));
-    enqueue_eval_tc(h, h->beta_mc, h->p, C, nullptr);
+    enqueue_eval_tc(h, h->beta, h->p, C, nullptr);
     cudaStreamSynchronize(h->stream);
     cudaMemcpy(tl.data(), h->dbg_time, tl.size() * sizeof(long long), cudaMemcpyDeviceToHost);
     cudaFree(h->dbg_time);
@@ -1551,14 +1552,12 @@ int grow(lrb_handle* h, double** buf, size_t* cap, size_t need) {
   return LRB_OK;
 }
 
-SamplerState* run_states(lrb_handle* h) { return h->run_C > 1 ? h->states_mc : h->state; }
-
 // one evaluation of every chain of the armed run at its state's beta_in
 int enqueue_run_eval(lrb_handle* h) {
   if (h->run_C > 1)
-    return enqueue_eval_mc(h, h->states_mc->beta_in, (long long)(sizeof(SamplerState) / sizeof(double)),
-                           h->run_C, h->states_mc);
-  return enqueue_eval(h, h->state->beta_in, h->state, h->run_want_grad);
+    return enqueue_eval_mc(h, h->states->beta_in, (long long)(sizeof(SamplerState) / sizeof(double)),
+                           h->run_C, h->states);
+  return enqueue_eval(h, h->states->beta_in, h->states, h->run_want_grad);
 }
 
 // capture `nodes` consecutive evaluations into an executable graph
@@ -1609,7 +1608,7 @@ int arm_run(lrb_handle* h, const lrb_sampler_params* params, const double* init,
   const int p = h->p;
   const long long steps = thin * iters;
   int rc;
-  if (C > 1 && (rc = ensure_chains(h, C))) return rc;
+  if ((rc = ensure_chains(h, C))) return rc;
   if (C > 1 && (rc = reserve_tc(h, C))) return rc;
   const bool want_moments = (params->flags & LRB_RUN_MOMENTS) != 0;
   const bool no_samples = (params->flags & LRB_RUN_NO_SAMPLES) != 0;
@@ -1637,22 +1636,12 @@ int arm_run(lrb_handle* h, const lrb_sampler_params* params, const double* init,
   h->run_params.scale = nullptr;
   std::memcpy(h->pinned, params->scale, p * sizeof(double));
   CK(h, cudaMemcpyAsync(h->d_scale, h->pinned, p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  const double* d_init = nullptr;
-  if (init) {
-    if (C == 1) {
-      std::memcpy(h->pinned + kMaxP, init, p * sizeof(double));
-      CK(h, cudaMemcpyAsync(h->d_init, h->pinned + kMaxP, p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-      d_init = h->d_init;
-    } else {
-      CK(h, cudaMemcpyAsync(h->beta_mc, init, (size_t)C * p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-      d_init = h->beta_mc;
-    }
-  }
+  if (init) CK(h, cudaMemcpyAsync(h->beta, init, (size_t)C * p * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   // reuse the cached gradient / lpost of the paused chain when the caller vouches that init is its state
   const int reuse = (init && (params->flags & LRB_RUN_REUSE_CACHE) && h->chain_live && h->chain_kind == kind &&
                      h->chain_C == C && (kind == LRB_MALA || kind == LRB_HMC)) ? 1 : 0;
   h->run_C = C;
-  sampler_begin_kernel<<<C, kBlock, 0, h->stream>>>(run_states(h), d_init, h->d_scale, kind, params->l, p,
+  sampler_begin_kernel<<<C, kBlock, 0, h->stream>>>(h->states, init ? h->beta : nullptr, h->d_scale, kind, params->l, p,
                                                     params->rng, params->step, params->seed,
                                                     params->init_lpost, steps, thin, dz, du,
                                                     no_samples ? nullptr : h->d_out, reuse,
@@ -1690,7 +1679,7 @@ int launch_run(lrb_handle* h) {
   if (h->run_consumed) {
     // A repeated launch continues the chain: re-arm the window [t, t+steps) and
     // propose from the paused state (replayed draws, if any, start over).
-    sampler_begin_kernel<<<h->run_C, kBlock, 0, h->stream>>>(run_states(h), nullptr, h->d_scale, h->run_kind,
+    sampler_begin_kernel<<<h->run_C, kBlock, 0, h->stream>>>(h->states, nullptr, h->d_scale, h->run_kind,
                                                              h->run_params.l, h->p, h->run_params.rng,
                                                              h->run_params.step, h->run_params.seed, 0.0, steps,
                                                              h->run_thin, h->run_dz, h->run_du,
@@ -1709,7 +1698,7 @@ int launch_run(lrb_handle* h) {
     bool refused = false;
     while (needed > 0) {
       const int chunk = (int)std::min<long long>(needed, 1ll << 24);
-      int rc = enqueue_drive(h, h->state->beta_in, h->state, h->run_want_grad, chunk);
+      int rc = enqueue_drive(h, h->states->beta_in, h->states, h->run_want_grad, chunk);
       if (rc && h->drive_launch_failed && !h->chain_live_partial) { refused = true; break; }   // nothing ran yet: static path below
       if (rc) return rc;
       h->chain_live_partial = true;
@@ -1746,7 +1735,7 @@ int finish_run(lrb_handle* h, double* out, int64_t* accepted) {
     CK(h, cudaMemcpyAsync(out, h->d_out, cnt * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   std::vector<long long> acc(C, 0);
   std::vector<int> phase(C, -1);
-  SamplerState* st = run_states(h);
+  SamplerState* st = h->states;
   CK(h, cudaMemcpy2DAsync(acc.data(), sizeof(long long), &st->accepted, sizeof(SamplerState), sizeof(long long), C,
                           cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaMemcpy2DAsync(phase.data(), sizeof(int), &st->phase, sizeof(SamplerState), sizeof(int), C,
@@ -1792,7 +1781,7 @@ extern "C" int lrb_chain_state(lrb_handle* h, double* x, double* lpost, int64_t*
   if (!h->chain_live) return fail(h, LRB_E_STATE, "no chain has been run on this handle");
   if (use_device(h)) return LRB_E_CUDA;
   long long t = 0; double lp = 0.0;
-  SamplerState* st = h->chain_C > 1 ? h->states_mc : h->state;   // chain 0 of a many-chain run
+  SamplerState* st = h->states;   // chain 0 of a many-chain run
   if (x) CK(h, cudaMemcpyAsync(x, st->x, h->p * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaMemcpyAsync(&lp, &st->lp_x, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CK(h, cudaMemcpyAsync(&t, &st->t, sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
@@ -1847,8 +1836,7 @@ extern "C" int lrb_run_moments(lrb_handle* h, int pooled, int64_t* count, double
   CK(h, bc.alloc((size_t)rows * sizeof(long long)));
   CK(h, bm.alloc((size_t)rows * p * sizeof(double)));
   if (cov) CK(h, bv.alloc((size_t)rows * p * p * sizeof(double)));
-  SamplerState* st = C > 1 ? h->states_mc : h->state;
-  moments_out_kernel<<<rows, kBlock, 0, h->stream>>>(st, C, p, pooled ? 1 : 0, bc.as<long long>(), bm.as<double>(),
+  moments_out_kernel<<<rows, kBlock, 0, h->stream>>>(h->states, C, p, pooled ? 1 : 0, bc.as<long long>(), bm.as<double>(),
                                                      cov ? bv.as<double>() : nullptr);
   CK(h, cudaGetLastError());
   h->kernel_launches++;

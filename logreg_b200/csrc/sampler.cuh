@@ -574,14 +574,4 @@ __global__ void moments_out_kernel(const SamplerState* states, int C, int p, int
     }
 }
 
-// Separate finish launch (NCCL mode: runs after the allreduce of `sums`).
-__global__ void finish_kernel(FinishArgs f, const double* sums_global) {
-  __shared__ double sums[kMaxP + 1];
-  __shared__ double scratch[kWarps];
-  if (f.state && f.state->phase == PH_PAUSED) return;
-  for (int c = threadIdx.x; c <= f.p; c += kBlock) sums[c] = sums_global[c];
-  __syncthreads();
-  finish_eval(f, sums, scratch);
-}
-
 }  // namespace lrb

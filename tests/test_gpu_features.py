@@ -205,3 +205,40 @@ def test_many_chain_buffers_may_grow_between_runs(lr):
     m2, a2 = q.run_chains(k, inits, 1, 70, seed=9)
     np.testing.assert_array_equal(m2, m1)
     np.testing.assert_array_equal(a2, a1)
+
+
+@pytest.mark.parametrize("deterministic", [False, True], ids=["drive", "static"])
+def test_single_chain_survives_many_chain_buffer_growth(lr, deterministic):
+    """A single chain lives in row 0 of the per-chain buffers: growing them (eval_many with more
+    chains than ever before) must carry a paused chain, and a run armed with lrb_run_begin, over.
+    200 rows are one row batch, so drive mode's sums are exact too and the runs compare bit for bit."""
+    import ctypes as C
+    from logreg_b200 import _native as N
+
+    def chain(grow):
+        q = lr.Problem(deterministic=deterministic)
+        bt = q.gen_synthetic(200, 8, mode="fp32", seed=4)
+        sd = 2.2 / np.sqrt(200)
+        k = lr.malaKernel(q.lpost, q.glp, dt=(0.6 * sd) ** 2, pre=1.0)
+        kl = q.info()["kernel_launches"]
+        m1, a1 = q.run(k, bt, 1, 30, seed=7)
+        drive = q.info()["kernel_launches"] - kl == 2            # sampler_begin + one drive-mode launch
+        if grow:
+            q.eval_many(np.tile(bt, (16, 1)))
+        m2, a2 = q.run(k, None, 1, 30, seed=7)                     # continues the paused chain
+        sp = q._params(k, 7, N.RNG_PHILOX, -np.inf)
+        q._ck(q._lib.lrb_run_begin(q._h, C.byref(sp), None, 1, 30, None, None))
+        if grow:
+            q.eval_many(np.tile(bt, (40, 1)))
+        q._ck(q._lib.lrb_run_launch(q._h))
+        m3, a3 = np.empty((30, 8)), C.c_int64()
+        q._ck(q._lib.lrb_run_finish(q._h, N.as_dp(m3), C.byref(a3)))
+        return drive, [m1, m2, m3], [a1, a2, a3.value], q.chain_state()
+
+    (d_ref, m_ref, a_ref, st_ref), (d, m, a, st) = chain(False), chain(True)
+    assert d_ref == d == (not deterministic)
+    for got, ref in zip(m, m_ref):
+        np.testing.assert_array_equal(got, ref)
+    assert a == a_ref and sum(a) > 0
+    np.testing.assert_array_equal(st[0], st_ref[0])
+    assert st[1:] == st_ref[1:] and st[2] == 90
